@@ -2,7 +2,7 @@
 """bench.py -- amplitude-updates/s of the qubism state-vector hot path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload qft_rand|adder32|general] [--qubits n]
+                    [--workload qft_rand|adder32|general] [--qubits n] [--dump-outputs DIR]
 
 One STEP = one pass of the hot path over one batch of synthetic input: the whole primitive
 op stream of the workload circuit applied to an n-qubit device-resident state through the C
@@ -28,6 +28,13 @@ old value freed, QASM/Simulation.hs:94-122 -- then reductions and a readback, al
 timed region), roofline (HBM, for the fused-pass kernel, measured live with CUDA events on
 the launching stream), cpu_baseline (the oracle's C/OpenMP port on the host cores, bounded
 sample), clocks (nvidia-smi during the timed region).
+
+--dump-outputs DIR writes what the last timed step left in the state (a fixed, seeded sample of
+its amplitudes in index order, DIR/state.npy with their indices in DIR/state_index.npy) and what
+the last end-to-end step handed back (DIR/e2e_sumsq.npy, DIR/e2e_window.npy), all float64 with
+(re, im) in the last axis, 24 MiB at most.  The warm-up then always takes its longest length,
+so the timed steps start from the same state whatever the settling needed, and two builds can be
+compared output for output on the same arguments.
 
 --impl reference times the reference's CPU path.  The Haskell reference cannot be built here
 (no GHC) and its literal dense algorithm cannot reach 24 qubits on any machine (one gate
@@ -77,6 +84,30 @@ def inverse_ops(ops):
     """C^-1 for a stream of (near-)unitary U and CX ops: reversed, matrices conjugate-transposed."""
     import numpy as np
     return [op if op[0] == "CX" else ("U", op[1], np.asarray(op[2]).conj().T) for op in reversed(ops)]
+
+
+# ------------------------------------------------------------------------------ --dump-outputs
+DUMP_WINDOW, DUMP_WINDOWS = 4096, 256  # 2^20 amplitudes: 16 MiB of (re, im) pairs + 8 MiB of indices
+
+
+def state_sample(sv, n: int):
+    """The same seeded sample of the 2^n logical amplitudes whatever the build: DUMP_WINDOWS windows
+    of DUMP_WINDOW consecutive amplitudes (the whole state when it is smaller).  A collective on a
+    sharded state: every rank calls it."""
+    import numpy as np
+    w = min(DUMP_WINDOW, 1 << n)
+    nwin = (1 << n) // w
+    starts = np.sort(np.random.default_rng(0).choice(nwin, min(DUMP_WINDOWS, nwin), replace=False)) * w
+    amps = np.concatenate([sv.to_host(int(s), w) for s in starts])
+    index = (starts[:, None] + np.arange(w)).reshape(-1)
+    return {"state": amps.view(np.float64).reshape(-1, 2), "state_index": index.astype(np.float64)}
+
+
+def write_outputs(out_dir: str, arrays: dict):
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------ clocks
@@ -155,8 +186,8 @@ def cpu_sample_ops(n: int):
 
 
 def cpu_run(n: int, steps: int, warmup: int, budget_s: float = 150.0, keep_first: bool = False):
-    """Times the oracle's C/OpenMP port (one sweep per primitive op, no fusion) on the host.
-    Bounded: stops after `budget_s` seconds of timed work (at least one step)."""
+    """Times the oracle's C/OpenMP port (one sweep per primitive op, no fusion) on the host: `steps`
+    timed steps after at most `warmup` untimed ones (the warm-up stops after `budget_s` / 3 seconds)."""
     import numpy as np
     from oracle import cport
     cport.lib().sv_set_threads(cpu_threads())
@@ -172,21 +203,17 @@ def cpu_run(n: int, steps: int, warmup: int, budget_s: float = 150.0, keep_first
             first = v.copy()
         if time.perf_counter() - t_w > budget_s / 3:
             break
-    done = 0
     t0 = time.perf_counter()
     for _ in range(steps):
         cport.run_ops_inplace(n, packed, v)
-        done += 1
         if keep_first and first is None:
             first = v.copy()
-        if time.perf_counter() - t0 > budget_s:
-            break
     dt = time.perf_counter() - t0
     cores = int(cport.lib().sv_num_threads())
-    aups = len(ops) * (1 << n) * done / dt
+    aups = len(ops) * (1 << n) * steps / dt
     sample = (f"QFT-{n} + 2 random layers at n={n} ({len(ops)} primitive ops, {(16 << n) >> 20} MiB state), "
-              f"{done} step(s), one sweep per op, OpenMP x{cores}")
-    return aups, dt / done, cores, sample, done, first
+              f"{steps} step(s), one sweep per op, OpenMP x{cores}")
+    return aups, dt / steps, cores, sample, steps, first
 
 
 def literal_dense_sample():
@@ -220,7 +247,7 @@ def run_reference(args):
     if rank != 0:
         return
     os.environ["OMP_NUM_THREADS"] = str(cpu_threads())
-    aups, step_s, cores, sample, done, _ = cpu_run(CPU_SAMPLE_N, max(1, args.steps), args.warmup)
+    aups, step_s, cores, sample, done, _ = cpu_run(CPU_SAMPLE_N, args.steps, args.warmup)
     line = {
         "impl": "reference", "metric": METRIC, "value": aups, "unit": UNIT, "n_gpus": args.gpus, "steps": done,
         "warmup": args.warmup, "ms_per_step": step_s * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -320,8 +347,8 @@ def run_ours(args):
     # pass of every rank ran as a specialised kernel (sharded layouts take 6-10 steps to settle into
     # their cycle of period <= 6 and every structure of the cycle has to come round twice), at most
     # 32 more steps.  All ranks take the same number of steps (the steps hold collectives).
-    settle_steps, good, need = 0, 0, (2 if world == 1 else 6)
-    while ctx.get_option("jit") > 0 and good < need and settle_steps < 32:
+    settle_steps, good, need, max_settle = 0, 0, (2 if world == 1 else 6), 32
+    while ctx.get_option("jit") > 0 and good < need and settle_steps < max_settle:
         ctx.jit_wait()
         ctx.reset_stats()
         step()
@@ -330,6 +357,10 @@ def run_ours(args):
         ctx.sync()  # (the library's own collectives have drained before torch's all-reduce is enqueued)
         good = good + 1 if max_over_ranks(generic) == 0.0 else 0
         settle_steps += 1
+    if args.dump_outputs:
+        # the longest settling on every run: the timed steps start from the same state
+        for _ in range(max_settle - settle_steps):
+            step()
     barrier()
     mark(f"warm-up done ({settle_steps} settling steps)")
     ctx.reset_stats()
@@ -344,6 +375,7 @@ def run_ours(args):
     elapsed = e0.elapsed_time(e1) / 1e3
     st = ctx.stats()
     mark("timed steps done")
+    outputs = state_sample(sv, n) if args.dump_outputs else {}  # (before the steps below change the state)
     if world == 1 and elapsed < 1.5:
         # nvidia-smi samples every 100 ms: keep the same load running (outside the timed region,
         # after the counters were read) until it has seen at least 1.5 s of it
@@ -435,6 +467,9 @@ def run_ours(args):
     e2e_value = nops * float(1 << n) / e2e_dt
     h2d = 16 * shard + nops * 80
     d2h = 3 * 16 + 16 * win
+    if args.dump_outputs:
+        outputs["e2e_sumsq"] = np.array(red)  # (S0, S1) of qubits 0, n // 2, n - 1
+        outputs["e2e_window"] = w.view(np.float64).reshape(-1, 2)  # rank 0: the first `win` of its shard
 
     if rank != 0:
         if dist is not None:
@@ -551,6 +586,8 @@ def run_ours(args):
         line["round_trip"] = round_trip
     if cpu:
         line["cpu_baseline"] = cpu
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, outputs)
     print(json.dumps(line), flush=True)
     if dist is not None:
         dist.barrier()
@@ -567,7 +604,12 @@ def main():
     ap.add_argument("--qubits", type=int, default=0)
     ap.add_argument("--round-trip", action="store_true", help="also at 1 GPU: the untimed inverse-circuit check")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed (--impl ours)")
     args.warmup = max(args.warmup, 0)
     if args.impl == "reference":
         run_reference(args)
