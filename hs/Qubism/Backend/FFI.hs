@@ -9,6 +9,7 @@ mechanical on purpose; every binding is one line of the C header.
 module Qubism.Backend.FFI where
 
 import Data.Complex        (Complex)
+import Data.Int            (Int64)
 import Data.Word           (Word64)
 import Foreign.C.String    (CString)
 import Foreign.C.Types
@@ -51,3 +52,5 @@ foreign import ccall safe   "qb_dotc"            c_qb_dotc            :: Ptr QbS
 foreign import ccall safe   "qb_norm2"           c_qb_norm2           :: Ptr QbState -> Ptr CDouble -> IO CInt
 foreign import ccall safe   "qb_normalize"       c_qb_normalize       :: Ptr QbState -> IO CInt
 foreign import ccall safe   "qb_tensor"          c_qb_tensor          :: Ptr QbState -> Ptr QbState -> Ptr (Ptr QbState) -> IO CInt
+-- observables -----------------------------------------------------------------------------
+foreign import ccall safe   "qb_expect_pauli"    c_qb_expect_pauli    :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Int64 -> Ptr CDouble -> IO CInt

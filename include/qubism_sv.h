@@ -184,6 +184,20 @@ int qb_norm2(qb_state *s, double *out);                       /* LA.norm_2 (NOT 
 int qb_normalize(qb_state *s);                                /* normalize                */
 int qb_tensor(qb_state *a, qb_state *b, qb_state **out);      /* a `tensor` b             */
 
+/* ---- observables ----------------------------------------------------------------------- */
+/* Expectation values of Pauli strings: out[t] = realPart (sv <.> (P_t #> sv)), where P_t is the
+ * product of pauliX / pauliY / pauliZ (QGate.hs:90-108) on the qubits named by term t: bit q of
+ * xmask[t] / zmask[t] is REFERENCE qubit q; X = x only, Z = z only, Y = both, I = neither.
+ * Not normalised (the reference's <.> is not).  Observes the state (flushes it) and leaves its
+ * value unchanged.  Deterministic.  Distributed: a collective; every rank passes the same terms
+ * and receives all nterms values.
+ * Cost: one read-only sweep of the state per distinct X mask and 64 terms (counted in
+ * qb_stats.reduce_launches, two launches per sweep); a term whose X mask flips a qubit of known value
+ * (|0...0>, after a collapse) is exactly 0 and costs nothing.  Sharded: X / Y on global qubits first
+ * swap those qubits into the shard (QB_ERR_UNSUPPORTED if a string has X / Y on more qubits than a
+ * shard holds).  QB_ERR_ARG: a null pointer with nterms > 0, nterms < 0, a mask bit at or above n. */
+int qb_expect_pauli(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, int64_t nterms, double *out);
+
 /* ---- introspection (tests, bench, profiling) ------------------------------------------- */
 typedef struct {
   uint64_t ops_submitted;   /* primitive ops received through the ABI                     */

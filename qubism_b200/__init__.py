@@ -7,7 +7,7 @@ if libqubism_sv.so has not been built or no CUDA device is usable (there is no C
 from . import capi  # noqa: F401
 from .qgate import (QGate, apply, cnot, controlled, gate, hadamard, ident, ifBit, kronecker, onEvery, onJust,  # noqa: F401
                     onRange, pauliX, pauliY, pauliZ, unitary, unitary_matrix)
-from .statevec import (Context, StateVec, collapse, dimension, measure, measureQubit, mkQubit, mkStateVec,  # noqa: F401
-                       normalize, tensor, zero)
+from .statevec import (Context, StateVec, collapse, dimension, expectPauli, measure, measureQubit, mkQubit,  # noqa: F401
+                       mkStateVec, normalize, tensor, zero)
 
 __version__ = "0.1.0"

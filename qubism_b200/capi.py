@@ -90,6 +90,7 @@ SIGNATURES = {
     "qb_norm2": (_I, [_VP, C.POINTER(_D)]),
     "qb_normalize": (_I, [_VP]),
     "qb_tensor": (_I, [_VP, _VP, C.POINTER(_VP)]),
+    "qb_expect_pauli": (_I, [_VP, C.POINTER(_U64), C.POINTER(_U64), _I64, C.POINTER(_D)]),
     "qb_get_stats": (_I, [_VP, C.POINTER(QbStats)]),
     "qb_reset_stats": (_I, [_VP]),
     "qb_ctx_stream": (_VP, [_VP]),

@@ -10,6 +10,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <map>
 #include <memory>
 #include <mutex>
 #include <string>
@@ -57,9 +58,9 @@ struct qb_ctx {
   int sm_count = 148;
   cudaStream_t stream = nullptr;
   int rank = 0, nranks = 1, pbits = 0;
-  double *red_partials = nullptr;  // device, 2 * max blocks
-  double *red_out = nullptr;       // device, 2 doubles (+2 spare)
-  double *red_host = nullptr;      // pinned, 4 doubles
+  double *red_partials = nullptr;  // device, kExpMaxTerms per block of the largest reduction grid
+  double *red_out = nullptr;       // device, kExpMaxTerms doubles
+  double *red_host = nullptr;      // pinned, kExpMaxTerms doubles
   uint64_t jit_base_compiled = 0, jit_base_launches = 0;  // qb_reset_stats baselines of the process-wide counters
   double jit_base_ms = 0.0;
   int *kq_bits_dev = nullptr;      // 2 * QB_MAX_KQ ints
@@ -161,9 +162,9 @@ int init_common(qb_ctx *c) {
   c->sm_count = prop.multiProcessorCount;
   QB_CUDA(cudaStreamCreateWithFlags(&c->stream, cudaStreamNonBlocking));
   const int maxblocks = c->sm_count * 8 + 8;
-  QB_CUDA(cudaMalloc(&c->red_partials, sizeof(double) * 2 * maxblocks));
-  QB_CUDA(cudaMalloc(&c->red_out, sizeof(double) * 4));
-  QB_CUDA(cudaMallocHost(&c->red_host, sizeof(double) * 4));
+  QB_CUDA(cudaMalloc(&c->red_partials, sizeof(double) * kExpMaxTerms * maxblocks));
+  QB_CUDA(cudaMalloc(&c->red_out, sizeof(double) * kExpMaxTerms));
+  QB_CUDA(cudaMallocHost(&c->red_host, sizeof(double) * kExpMaxTerms));
   QB_CUDA(cudaMalloc(&c->kq_bits_dev, sizeof(int) * 2 * QB_MAX_KQ));
   QB_CUDA(cudaMalloc(&c->kq_mat_dev, sizeof(double2) << (2 * QB_MAX_KQ)));
   for (const char *name : {"tile_bits", "reg_bits", "low_bits", "max_rounds", "peephole", "fuse", "max_pass_gates", "l2_prefetch", "avoid_regswap", "hot_bits", "rot", "lite", "dbg_skip", "lane_fixed", "skip_dead", "support", "jit", "jit_group", "jit_pf_last", "jit_minb", "jit_mem", "tma", "oop", "oop_low_bits", "chunk_lanes", "oop_dist", "pf_lines", "fuse_exchange", "defer_tail"}) {
@@ -1839,6 +1840,121 @@ int qb_norm2(qb_state *s, double *out) {
   QB_TRY(materialise(s));
   QB_TRY(sumsq_buffer(s->b, -1, &s0, &s1));
   *out = std::sqrt(s0 + s1);
+  return QB_OK;
+}
+
+// ---- Pauli expectation values
+// Sharded states: an X / Y on a global qubit pairs amplitudes of two ranks, so the qubits of the logical
+// X mask lx are brought into the shard first.  One multi-bit swap through make_local; where its victims
+// carried one of those qubits out again (the victim choice knows only the qubits it brings in), a
+// relayout trades it for a local qubit outside lx.
+static int localise_x(Buffer *b, uint64_t lx) {
+  if (!(phys_mask(b, lx) >> b->L)) return QB_OK;
+  if (__builtin_popcountll(lx) > b->L)
+    return fail(QB_ERR_UNSUPPORTED, "a Pauli string with X / Y on %d qubits does not fit a shard of %d qubits",
+                __builtin_popcountll(lx), b->L);
+  std::vector<HostOp> ops;
+  for (uint64_t m = lx; m; m &= m - 1) {
+    HostOp h;
+    h.target = __builtin_ctzll(m);
+    ops.push_back(h);
+  }
+  std::vector<const HostOp *> pending;
+  for (const HostOp &h : ops) pending.push_back(&h);
+  QB_TRY(make_local(b, pending));
+  if (!(phys_mask(b, lx) >> b->L)) return QB_OK;
+  std::vector<int> want = b->perm, logical_of(b->n);
+  for (int q = 0; q < b->n; ++q) logical_of[want[q]] = q;
+  int spare = b->L - 1;  // highest local bit not holding a qubit of lx
+  for (uint64_t m = lx; m; m &= m - 1) {
+    const int q = __builtin_ctzll(m);
+    if (want[q] < b->L) continue;
+    while ((lx >> logical_of[spare]) & 1ull) --spare;  // (popc(lx) <= L: one is left)
+    const int o = logical_of[spare];
+    std::swap(want[q], want[o]);
+    logical_of[want[q]] = q;
+    logical_of[want[o]] = o;
+  }
+  return relayout(b, want);
+}
+
+int qb_expect_pauli(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, int64_t nterms, double *out) {
+  if (!s) return fail(QB_ERR_ARG, "null state");
+  if (nterms < 0) return fail(QB_ERR_ARG, "nterms %lld < 0", (long long)nterms);
+  if (nterms == 0) return QB_OK;
+  if (!xmask || !zmask || !out) return fail(QB_ERR_ARG, "null argument");
+  const int n = s->n;
+  for (int64_t t = 0; t < nterms; ++t)
+    if ((xmask[t] | zmask[t]) >> n) return fail(QB_ERR_ARG, "term %lld names a qubit >= %d", (long long)t, n);
+  qb_ctx *c = s->ctx;
+  Guard g(c);
+  QB_TRY(materialise(s));
+  Buffer *b = s->b;
+  if (!(std::isfinite(b->pscale[0]) && std::isfinite(b->pscale[1]))) QB_TRY(force_scale(b));  // NaN / inf must reach the data
+  auto logical = [n](uint64_t m) {  // reference qubit q is logical bit n - 1 - q
+    uint64_t r = 0;
+    for (; m; m &= m - 1) r |= 1ull << (n - 1 - __builtin_ctzll(m));
+    return r;
+  };
+  std::vector<uint64_t> lx(nterms), lz(nterms);
+  std::map<uint64_t, std::vector<int64_t>> groups;  // logical X mask -> its terms in caller order (same on every rank)
+  for (int64_t t = 0; t < nterms; ++t) {
+    lx[t] = logical(xmask[t]);
+    lz[t] = logical(zmask[t]);
+    out[t] = 0.0;
+    // an X on a qubit of known value pairs every non-zero amplitude with a zero one: exactly 0
+    if (c->opt.support && (lx[t] & b->zmask)) continue;
+    groups[lx[t]].push_back(t);
+  }
+  const double g2 = b->pscale[0] * b->pscale[0] + b->pscale[1] * b->pscale[1];  // the pending scalar, arithmetically
+  const uint64_t local = (1ull << b->L) - 1ull;
+  for (const auto &grp : groups) {
+    const uint64_t x = grp.first;
+    const std::vector<int64_t> &terms = grp.second;
+    if (c->nranks > 1) QB_TRY(localise_x(b, x));
+    const uint64_t xp = phys_mask(b, x);
+    const uint64_t lo = xp ? (1ull << (63 - __builtin_clzll(xp))) - 1ull : ~0ull;
+    for (size_t k0 = 0; k0 < terms.size(); k0 += kExpMaxTerms) {
+      const size_t k1 = std::min(terms.size(), k0 + size_t(kExpMaxTerms));
+      ExpTerms et;
+      memset(&et, 0, sizeof et);
+      et.xp = xp;
+      et.lo_mask = lo;
+      int64_t order[kExpMaxTerms];
+      double post[kExpMaxTerms];
+      for (int odd = 0; odd < 2; ++odd)  // real parts (even popc(x & z)) first
+        for (size_t k = k0; k < k1; ++k)
+          if ((__builtin_popcountll(x & lz[terms[k]]) & 1) == odd) order[et.nterms++] = terms[k];
+      for (int j = 0; j < et.nterms; ++j) {
+        const int64_t t = order[j];
+        const int ph = __builtin_popcountll(x & lz[t]) & 3;  // P = i^ph X^x Z^z (Y = i X Z)
+        if (!(ph & 1)) et.neven = j + 1;
+        const uint64_t zp = phys_mask(b, lz[t]);
+        et.zp[j] = zp & local;
+        for (uint32_t u = 0; u < (uint32_t)kExpU; ++u) {
+          const uint64_t p = uint64_t(u) << kExpUShift, i = (p & lo) | ((p & ~lo) << 1);
+          if (__builtin_popcountll(i & et.zp[j]) & 1) et.rflip[j] |= 1u << u;
+        }
+        // Re(i^ph (w + (-1)^ph conj w)) = 2 * (+1, -1, -1, +1)[ph] * (Re w | Im w) over a pair; one
+        // amplitude (xp == 0) counts once.  Z on global qubits: this rank's value of them
+        double f = (ph == 1 || ph == 2) ? -1.0 : 1.0;
+        if (xp) f *= 2.0;
+        if (__builtin_popcountll((zp >> b->L) & uint64_t(c->rank)) & 1) f = -f;
+        post[j] = f;
+      }
+      QB_CUDA(launch_expect_pauli(b->amps, b->L, et, c->red_partials, c->red_out, c->sm_count, c->stream));
+      c->stats.reduce_launches += 2;
+      QB_CUDA(cudaMemcpyAsync(c->red_host, c->red_out, sizeof(double) * et.nterms, cudaMemcpyDeviceToHost, c->stream));
+      QB_CUDA(cudaStreamSynchronize(c->stream));
+      double v[kExpMaxTerms];
+      for (int j = 0; j < et.nterms; ++j) v[j] = c->red_host[j] * post[j];
+      if (c->nranks > 1) {
+        int rc = dist_allreduce_sum(c->dist, v, et.nterms, c->stream);
+        if (rc != QB_OK) return fail(rc, "allreduce failed: %s", dist_last_error());
+      }
+      for (int j = 0; j < et.nterms; ++j) out[order[j]] = g2 != 1.0 ? v[j] * g2 : v[j];
+    }
+  }
   return QB_OK;
 }
 

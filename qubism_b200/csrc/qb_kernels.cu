@@ -1124,6 +1124,92 @@ cudaError_t launch_dotc(const double2 *a, const double2 *b, uint64_t n, double *
   return cudaGetLastError();
 }
 
+// ---------------------------------------------------------------- Pauli expectation values
+// One launch = one group of terms sharing the physical X mask xp.  With h = the top bit of xp, every
+// index i with bit h clear meets its partner j = i ^ xp once; the pair product w = conj(psi_j) psi_i is
+// formed once and each term adds (-1)^popc(i & zp) times Re w (even popc(x & z)) or Im w (odd); the host
+// applies the factor 2, the phase sign and the global-qubit signs.  xp == 0: every i, w = |psi_i|^2.
+// A thread takes kExpU pairs per step, pair numbers p0 + u * kRedThreads: the bits of u are a field of
+// their own in p, so popc(i_u & zp) = popc(i_0 & zp) + popc(ins(u << 8) & zp), and the second part is
+// the host-made bit u of ExpTerms::rflip.  Per term and step one POPC; per term and pair a few integer
+// instructions (the sign goes straight into the high word) and one DADD.
+static_assert(kRedThreads == 1 << kExpUShift, "ExpTerms::rflip: u is the pair-number field above the thread index");
+
+__global__ void __launch_bounds__(kRedThreads) k_expect_final(const double *__restrict__ partials, int nblocks, int stride,
+                                                             double *__restrict__ out) {
+  double acc[1] = {0.0};
+  for (int i = threadIdx.x; i < nblocks; i += kRedThreads) acc[0] += partials[size_t(i) * stride + blockIdx.x];
+  block_reduce_store<1>(acc, out + blockIdx.x);
+}
+
+template <int NT>
+__global__ void __launch_bounds__(kRedThreads, NT >= 16 ? 1 : 4) k_expect_pauli_partial(const double2 *__restrict__ amps, uint64_t npairs,
+                                                                     const __grid_constant__ ExpTerms terms,
+                                                                     double *__restrict__ partials) {
+  double acc[NT];
+#pragma unroll
+  for (int t = 0; t < NT; ++t) acc[t] = 0.0;
+  const uint64_t lo = terms.lo_mask, xp = terms.xp;
+  const uint64_t stride = uint64_t(gridDim.x) * (kRedThreads * kExpU);
+  for (uint64_t p0 = blockIdx.x * uint64_t(kRedThreads * kExpU) + threadIdx.x; p0 < npairs; p0 += stride) {
+    double re[kExpU], im[kExpU];
+    const uint64_t i0 = (p0 & lo) | ((p0 & ~lo) << 1);
+#pragma unroll
+    for (int u = 0; u < kExpU; ++u) {
+      const uint64_t p = p0 + uint64_t(u) * kRedThreads;
+      re[u] = im[u] = 0.0;
+      if (p < npairs) {
+        const uint64_t i = (p & lo) | ((p & ~lo) << 1);  // bit h inserted (lo_mask = ~0: none)
+        const double2 a = __ldcs(amps + i);
+        if (xp) {
+          const double2 b = __ldcs(amps + (i ^ xp));
+          re[u] = __dadd_rn(__dmul_rn(b.x, a.x), __dmul_rn(b.y, a.y));
+          im[u] = __dsub_rn(__dmul_rn(b.x, a.y), __dmul_rn(b.y, a.x));
+        } else {
+          re[u] = __dadd_rn(__dmul_rn(a.x, a.x), __dmul_rn(a.y, a.y));
+        }
+      }
+    }
+#pragma unroll
+    for (int t = 0; t < NT; ++t) {
+      const uint32_t base = (0u - (uint32_t(__popcll(i0 & terms.zp[t])) & 1u)) ^ terms.rflip[t];
+#pragma unroll
+      for (int u = 0; u < kExpU; ++u) {
+        const double v = t < terms.neven ? re[u] : im[u];
+        const int hi = __double2hiint(v) ^ int((base << (31 - u)) & 0x80000000u);
+        acc[t] = __dadd_rn(acc[t], __hiloint2double(hi, __double2loint(v)));
+      }
+    }
+  }
+  block_reduce_store<NT>(acc, partials + size_t(NT) * blockIdx.x);
+}
+
+template <int NT>
+static cudaError_t expect_launch(const double2 *amps, uint64_t npairs, const ExpTerms &terms, double *partials_dev,
+                                 double *out_dev, int sm_count, cudaStream_t stream) {
+  int per_sm = 0;
+  cudaError_t e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_expect_pauli_partial<NT>, kRedThreads, 0);
+  if (e != cudaSuccess) return e;
+  const int g = grid_for(npairs, kRedThreads * kExpU, sm_count, std::max(1, std::min(per_sm, 8)));
+  k_expect_pauli_partial<NT><<<g, kRedThreads, 0, stream>>>(amps, npairs, terms, partials_dev);
+  // partials[block][NT]: one block of the final stage per term
+  k_expect_final<<<terms.nterms, kRedThreads, 0, stream>>>(partials_dev, g, NT, out_dev);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_expect_pauli(const double2 *amps, int local_bits, const ExpTerms &terms, double *partials_dev,
+                                double *out_dev, int sm_count, cudaStream_t stream) {
+  if (terms.nterms < 1 || terms.nterms > kExpMaxTerms || terms.neven > terms.nterms) return cudaErrorInvalidValue;
+  const uint64_t npairs = terms.xp ? (1ull << (local_bits - 1)) : (1ull << local_bits);
+  if (terms.nterms <= 1) return expect_launch<1>(amps, npairs, terms, partials_dev, out_dev, sm_count, stream);
+  if (terms.nterms <= 2) return expect_launch<2>(amps, npairs, terms, partials_dev, out_dev, sm_count, stream);
+  if (terms.nterms <= 4) return expect_launch<4>(amps, npairs, terms, partials_dev, out_dev, sm_count, stream);
+  if (terms.nterms <= 8) return expect_launch<8>(amps, npairs, terms, partials_dev, out_dev, sm_count, stream);
+  if (terms.nterms <= 16) return expect_launch<16>(amps, npairs, terms, partials_dev, out_dev, sm_count, stream);
+  if (terms.nterms <= 32) return expect_launch<32>(amps, npairs, terms, partials_dev, out_dev, sm_count, stream);
+  return expect_launch<64>(amps, npairs, terms, partials_dev, out_dev, sm_count, stream);
+}
+
 // ---------------------------------------------------------------- live sub-cube kernels
 // After a collapse (StateVec.hs:104-114) half of the state is exactly zero, and a fresh
 // |0...0> is zero outside one amplitude.  The host tracks the index bits whose value is KNOWN

@@ -38,6 +38,23 @@ cudaError_t launch_sumsq(const double2 *amps, uint64_t n, int bit, double *parti
 cudaError_t launch_dotc(const double2 *a, const double2 *b, uint64_t n, double *partials_dev, double *out_dev,
                         int sm_count, cudaStream_t stream);
 
+// Expectation values of up to kExpMaxTerms Pauli strings that share one X mask, in one read-only sweep
+// (qb_expect_pauli).  out_dev[t] = sum over the pairs (i, i ^ xp), bit h of i clear (h = top bit of xp), of
+// (-1)^popc(i & zp[t]) * (t < neven ? Re : Im) conj(amps[i ^ xp]) amps[i]; xp == 0: sum over every i of
+// (-1)^popc(i & zp[t]) |amps[i]|^2.  Deterministic (fixed grid per device, fixed-order two-stage sum).
+constexpr int kExpMaxTerms = 64;
+constexpr int kExpU = 4;          // pairs per thread and step: pair numbers p0 + u * 256 (u at bit kExpUShift)
+constexpr int kExpUShift = 8;
+struct ExpTerms {
+  uint64_t xp;       // physical X mask (local bits)
+  uint64_t lo_mask;  // bits below h ((1 << h) - 1); ~0 when xp == 0
+  int32_t nterms, neven;
+  uint64_t zp[kExpMaxTerms];     // physical Z mask (local bits) per term
+  uint32_t rflip[kExpMaxTerms];  // bit u: popc(deposit(u << kExpUShift) & zp[t]) is odd (deposit = insert a 0 at bit h)
+};
+cudaError_t launch_expect_pauli(const double2 *amps, int local_bits, const ExpTerms &terms, double *partials_dev,
+                                double *out_dev, int sm_count, cudaStream_t stream);
+
 // Live sub-cube {i : i & fixed_mask == fixed_val} of the shard (see "support" in qb_api.cpp): the
 // reduction of launch_sumsq restricted to it, and zero-fill (mode 0) / scaling (mode 1) of it.
 int cube_runs(int local_bits, uint64_t fixed_mask);  // must be <= kMaxRuns for the launchers below

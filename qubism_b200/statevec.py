@@ -301,6 +301,19 @@ class StateVec:
         capi.check(self.ctx.L.qb_dotc(self._h, other._h, C.byref(out)))
         return complex(out.re, out.im)
 
+    def expect_pauli(self, terms) -> np.ndarray:
+        """``realPart (sv <.> (p #> sv))`` for each Pauli string ``p`` of ``terms`` (qb_expect_pauli), in one
+        read-only sweep per distinct X mask; the state is not normalised first and keeps its value.
+        A term is a string over ``IXYZ`` of length n (character q acts on qubit q) or an
+        ``(xmask, zmask)`` pair (bit q = qubit q; X: x only, Z: z only, Y: both).  Returns float64[len(terms)]."""
+        n = self.n
+        xs, zs = pauli_masks(terms, n)
+        out = np.zeros(len(xs), dtype=np.float64)
+        P64 = C.POINTER(C.c_uint64)
+        capi.check(self.ctx.L.qb_expect_pauli(self._h, xs.ctypes.data_as(P64), zs.ctypes.data_as(P64), len(xs),
+                                              out.ctypes.data_as(C.POINTER(C.c_double))))
+        return out
+
     def norm(self) -> float:  # Algebra.hs:35-36: realPart (a <.> a), the SQUARED norm
         return self.inner(self).real
 
@@ -310,6 +323,22 @@ class StateVec:
         return (self - other).norm2() < 0.000001
 
     __hash__ = None
+
+
+def pauli_masks(terms, n: int):
+    """Pauli strings (``"XIZY"``, character q = qubit q) or ``(xmask, zmask)`` pairs -> two uint64 arrays."""
+    xs, zs = [], []
+    for term in terms:
+        if isinstance(term, str):
+            if len(term) != n or any(ch not in "IXYZ" for ch in term.upper()):
+                raise ValueError(f"Pauli string {term!r}: want {n} characters of IXYZ")
+            x = sum(1 << q for q, ch in enumerate(term.upper()) if ch in "XY")
+            z = sum(1 << q for q, ch in enumerate(term.upper()) if ch in "ZY")
+        else:
+            x, z = (int(m) for m in term)
+        xs.append(x)
+        zs.append(z)
+    return np.array(xs, dtype=np.uint64), np.array(zs, dtype=np.uint64)
 
 
 # ---- module-level functions with the reference's names (StateVec.hs:14-25) -----------------
@@ -361,3 +390,8 @@ def measureQubit(i: int, sv: StateVec, r: float) -> int:
 def measure(sv: StateVec, rs) -> list:
     """StateVec.hs:133-137."""
     return sv.measure_(rs)
+
+
+def expectPauli(terms, sv: StateVec) -> np.ndarray:
+    """``[realPart (sv <.> (p #> sv)) | p <- terms]`` without building any ``p #> sv`` (see StateVec.expect_pauli)."""
+    return sv.expect_pauli(terms)
