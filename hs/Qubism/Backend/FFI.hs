@@ -54,3 +54,5 @@ foreign import ccall safe   "qb_normalize"       c_qb_normalize       :: Ptr QbS
 foreign import ccall safe   "qb_tensor"          c_qb_tensor          :: Ptr QbState -> Ptr QbState -> Ptr (Ptr QbState) -> IO CInt
 -- observables -----------------------------------------------------------------------------
 foreign import ccall safe   "qb_expect_pauli"    c_qb_expect_pauli    :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Int64 -> Ptr CDouble -> IO CInt
+-- Pauli rotations ------------------------------------------------------------------------
+foreign import ccall safe   "qb_apply_pauli_rot" c_qb_apply_pauli_rot :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Ptr CDouble -> Int64 -> IO CInt

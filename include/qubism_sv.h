@@ -198,6 +198,23 @@ int qb_tensor(qb_state *a, qb_state *b, qb_state **out);      /* a `tensor` b   
  * shard holds).  QB_ERR_ARG: a null pointer with nterms > 0, nterms < 0, a mask bit at or above n. */
 int qb_expect_pauli(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, int64_t nterms, double *out);
 
+/* ---- Pauli rotations ------------------------------------------------------------------- */
+/* s <- R_{P_t}(theta[t]) ... R_{P_0}(theta[0]) s, with R_P(theta) = exp(-i theta/2 P)
+ * = cos(theta/2) I - i sin(theta/2) P and P_t named by xmask[t] / zmask[t] exactly as in
+ * qb_expect_pauli (bit q = REFERENCE qubit q; X = x only, Z = z only, Y = both; pauliY as in
+ * QGate.hs:90-108).  Applied in array order.  Enqueues only, like every gate call; the identity
+ * string is a global factor exp(-i theta/2) and launches nothing.
+ * Cost: one read + write sweep of the state (counted in qb_stats.simple_launches) per run of
+ * consecutive rotations whose X qubits fit one tile of QB_PAULI_ROT_MAX_X qubits together, at most 64
+ * rotations each; Z-only rotations fit any run.  A run ends the fused pass before it.  Sharded: X / Y on
+ * global qubits first swap those qubits into the shard.
+ * Checked before anything is queued (a rejected call leaves the state and its queue untouched):
+ * QB_ERR_ARG: a null pointer with nrot > 0, nrot < 0, a mask bit at or above n, a non-finite theta.
+ * QB_ERR_UNSUPPORTED: a string with X / Y on more than QB_PAULI_ROT_MAX_X qubits, or on more
+ * qubits than a shard holds. */
+#define QB_PAULI_ROT_MAX_X 12
+int qb_apply_pauli_rot(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, const double *theta, int64_t nrot);
+
 /* ---- introspection (tests, bench, profiling) ------------------------------------------- */
 typedef struct {
   uint64_t ops_submitted;   /* primitive ops received through the ABI                     */

@@ -91,6 +91,7 @@ SIGNATURES = {
     "qb_normalize": (_I, [_VP]),
     "qb_tensor": (_I, [_VP, _VP, C.POINTER(_VP)]),
     "qb_expect_pauli": (_I, [_VP, C.POINTER(_U64), C.POINTER(_U64), _I64, C.POINTER(_D)]),
+    "qb_apply_pauli_rot": (_I, [_VP, C.POINTER(_U64), C.POINTER(_U64), C.POINTER(_D), _I64]),
     "qb_get_stats": (_I, [_VP, C.POINTER(QbStats)]),
     "qb_reset_stats": (_I, [_VP]),
     "qb_ctx_stream": (_VP, [_VP]),

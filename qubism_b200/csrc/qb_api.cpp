@@ -85,12 +85,14 @@ struct qb_ctx {
 };
 
 // One entry of a lineage log: what a handle did after the position its buffer stands at.
-enum LogKind : int { LOG_1Q = 0, LOG_KQ = 2, LOG_SCALE = 3, LOG_COLLAPSE = 4 };
+enum LogKind : int { LOG_1Q = 0, LOG_KQ = 2, LOG_SCALE = 3, LOG_COLLAPSE = 4, LOG_PAULI = 5 };
 struct LogOp {
   int kind = LOG_1Q;
   int target = -1;    // 1Q: logical target bit.  COLLAPSE: the logical bit
-  uint64_t ctrl = 0;  // 1Q / KQ: logical control mask.  COLLAPSE: the outcome (0 / 1)
-  double m[8] = {0};  // 1Q: the matrix.  SCALE: (re, im).  COLLAPSE: m[0] = weight of the outcome
+  uint64_t ctrl = 0;  // 1Q / KQ: logical control mask.  COLLAPSE: the outcome (0 / 1).  PAULI: logical X mask
+  uint64_t pz = 0;    // PAULI: logical Z mask
+  double m[8] = {0};  // 1Q: the matrix.  SCALE: (re, im).  COLLAPSE: m[0] = weight of the outcome.
+                      // PAULI: (cos(theta/2), sin(theta/2))
   int k = 0;
   int kq_bits[QB_MAX_KQ] = {0};
   std::shared_ptr<const std::vector<double>> kq_m;
@@ -147,6 +149,10 @@ struct qb_state {
   int n = 0;
   bool stale = false;  // option "linear": a later pure application consumed this value
 };
+
+extern "C" {
+static int localise_x(Buffer *b, uint64_t lx);  // (with the Pauli expectation values, below)
+}
 
 namespace {
 
@@ -842,7 +848,9 @@ int run_fused_segment(Buffer *s, std::vector<const HostOp *> seg, const double *
 // what one executed op does to the support.  Applied right after the op has run: the NEXT
 // segment of the same flush plans its dead tiles from it (a dense block populates its qubits).
 void support_after_op(Buffer *s, const HostOp &op) {
-  if (op.kind == 2) {
+  if (op.kind == 3) {  // (a Z-only rotation is a phase: what is zero stays zero)
+    s->zmask &= ~op.px;
+  } else if (op.kind == 2) {
     for (int j = 0; j < op.k; ++j) s->zmask &= ~(1ull << op.kq_bits[j]);
     for (double x : op.kq_m)
       if (!std::isfinite(x)) {
@@ -857,6 +865,75 @@ void support_after_op(Buffer *s, const HostOp &op) {
     if (op.type != G_DIAG) s->zmask &= ~(1ull << op.target);
   }
   s->zval &= s->zmask;
+}
+
+// A stretch of consecutive Pauli rotations (HostOp kind 3), cut greedily into launches of k_pauli_rot_tile
+// (one read + write sweep each).  A rotation joins the running launch while that holds fewer than
+// kPauliMaxRot and its X qubits add nothing to the launch's X union or the union with the three low
+// physical bits (one 128-byte line) still fits the tile; the tile is that union topped up with the lowest
+// other local bits.  Sharded: the launch's X qubits are brought into the shard first, and Z on global qubits
+// becomes this rank's sign.
+static_assert(kPauliTileBits == QB_PAULI_ROT_MAX_X, "the tile holds the widest string the header allows");
+int run_pauli_rots(Buffer *s, const std::vector<const HostOp *> &run) {
+  qb_ctx *c = s->ctx;
+  QB_TRY(ensure_inplace(s));
+  const int L = s->L, T = std::min(kPauliTileBits, L);
+  const uint64_t local = (1ull << L) - 1ull, low = (1ull << std::min(3, L)) - 1ull;
+  for (size_t i0 = 0; i0 < run.size();) {
+    uint64_t ux = 0;  // logical X union of the launch
+    size_t i1 = i0;
+    for (; i1 < run.size() && i1 - i0 < size_t(kPauliMaxRot); ++i1) {
+      const uint64_t x = run[i1]->px;
+      if (i1 > i0 && (x & ~ux) && __builtin_popcountll(phys_mask(s, ux | x) | low) > T) break;
+      ux |= x;
+    }
+    if (c->nranks > 1) QB_TRY(localise_x(s, ux));
+    uint64_t tile = phys_mask(s, ux);
+    if (__builtin_popcountll(tile) > T || (tile & ~local))
+      return fail(QB_ERR_UNSUPPORTED, "internal: Pauli rotations with X outside the rotation tile");
+    for (int b = 0; __builtin_popcountll(tile) < T; ++b) tile |= 1ull << b;
+    PauliRotArgs args;
+    memset(&args, 0, sizeof args);
+    args.nrot = uint32_t(i1 - i0);
+    args.tile_bits = uint32_t(T);
+    for (int b = 0, i = 0; b < L; ++b)
+      if ((tile >> b) & 1ull) args.tile_pos[i++] = uint8_t(b);
+    for (int b = 0; b < L;) {  // runs of the local bits outside the tile
+      if ((tile >> b) & 1ull) {
+        ++b;
+        continue;
+      }
+      int e = b;
+      while (e < L && !((tile >> e) & 1ull)) ++e;
+      args.run_shift[args.nruns] = uint8_t(b);
+      args.run_len[args.nruns++] = uint8_t(e - b);
+      b = e;
+    }
+    auto tile_local = [&](uint64_t m) {
+      uint32_t r = 0;
+      for (int i = 0; i < T; ++i) r |= uint32_t((m >> args.tile_pos[i]) & 1ull) << i;
+      return r;
+    };
+    for (size_t i = i0; i < i1; ++i) {
+      const HostOp &h = *run[i];
+      const uint64_t xp = phys_mask(s, h.px), zp = phys_mask(s, h.pz);
+      PauliRotParam &p = args.rot[i - i0];
+      p.xt = tile_local(xp);
+      p.zt = tile_local(zp);
+      p.zout = zp & local & ~tile;
+      p.c = h.m[0];
+      // the partner's factor -i s i^ph, ph = popc(x & z) mod 4 (P = i^ph X^x Z^z: Y = i X Z)
+      const double f = (__builtin_popcountll((zp >> L) & uint64_t(c->rank)) & 1) ? -h.m[1] : h.m[1];
+      const int ph = __builtin_popcountll(h.px & h.pz) & 3;
+      p.ar = ph == 1 ? f : ph == 3 ? -f : 0.0;
+      p.ai = ph == 0 ? -f : ph == 2 ? f : 0.0;
+    }
+    QB_CUDA(launch_pauli_rot(s->amps, L, args, c->stream));
+    c->stats.simple_launches++;
+    c->stats.ops_executed += args.nrot;
+    i0 = i1;
+  }
+  return QB_OK;
 }
 
 // run the queued ops.  The deferred scalar rides on the last fused pass if there is one;
@@ -902,10 +979,26 @@ int exec_queue(Buffer *s) {
       if (s->perm[op.kq_bits[j]] >= s->L) return true;
     return false;
   };
+  // the stretch of consecutive Pauli rotations that starts at op i; i moves to its last op
+  auto pauli_stretch = [&](size_t &i) {
+    std::vector<const HostOp *> run;
+    size_t j = i;
+    for (; j < q.ops.size() && (q.ops[j].dead || q.ops[j].kind == 3); ++j)
+      if (!q.ops[j].dead) run.push_back(&q.ops[j]);
+    i = j - 1;
+    const int r = run_pauli_rots(s, run);
+    if (r == QB_OK)
+      for (const HostOp *h : run) support_after_op(s, *h);
+    return r;
+  };
   if (T == 0) {
     for (size_t i = 0; i < q.ops.size(); ++i) {
       const HostOp &op = q.ops[i];
       if (op.dead) continue;
+      if (op.kind == 3) {
+        if ((rc = pauli_stretch(i)) != QB_OK) break;
+        continue;
+      }
       if ((op.kind == 0 && op.type != G_DIAG && s->perm[op.target] >= s->L) || (op.kind == 2 && kq_needs_swap(op)))
         if ((rc = make_local(s, pending_from(i))) != QB_OK) break;
       if ((rc = run_simple(s, op)) != QB_OK) break;
@@ -923,6 +1016,10 @@ int exec_queue(Buffer *s) {
       if (!seg.empty()) {
         rc = run_fused_segment(s, seg, nullptr, nullptr);
         seg.clear();
+      }
+      if (op.kind == 3) {  // (ends the fused segment, as a dense block does)
+        if (rc == QB_OK) rc = pauli_stretch(i);
+        continue;
       }
       if (rc == QB_OK && kq_needs_swap(op)) rc = make_local(s, pending_from(i));
       if (rc == QB_OK) rc = run_simple(s, op);
@@ -1079,6 +1176,7 @@ int exec_log(Buffer *b, size_t upto) {
       case LOG_1Q: b->q.push_1q(o.target, o.ctrl, o.m); break;
       case LOG_KQ: b->q.push_kq(o.kq_bits, o.k, o.kq_m->data(), o.ctrl); break;
       case LOG_SCALE: b->q.mul_gscale(o.m[0], o.m[1]); break;
+      case LOG_PAULI: b->q.push_pauli(o.ctrl, o.pz, o.m[0], o.m[1]); break;
       case LOG_COLLAPSE:
         rc = exec_queue(b);
         if (rc == QB_OK) rc = collapse_exec(b, o.target, (int)o.ctrl, o.m[0]);
@@ -1954,6 +2052,39 @@ int qb_expect_pauli(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, i
       }
       for (int j = 0; j < et.nterms; ++j) out[order[j]] = g2 != 1.0 ? v[j] * g2 : v[j];
     }
+  }
+  return QB_OK;
+}
+
+// ---- Pauli rotations
+int qb_apply_pauli_rot(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, const double *theta, int64_t nrot) {
+  if (!s) return fail(QB_ERR_ARG, "null state");
+  if (nrot < 0) return fail(QB_ERR_ARG, "nrot %lld < 0", (long long)nrot);
+  if (nrot == 0) return QB_OK;
+  if (!xmask || !zmask || !theta) return fail(QB_ERR_ARG, "null argument");
+  const int n = s->n, T = std::min(kPauliTileBits, s->n - s->ctx->pbits);
+  for (int64_t t = 0; t < nrot; ++t) {  // everything is checked before anything is queued
+    if ((xmask[t] | zmask[t]) >> n) return fail(QB_ERR_ARG, "rotation %lld names a qubit >= %d", (long long)t, n);
+    if (!std::isfinite(theta[t])) return fail(QB_ERR_ARG, "rotation %lld: theta is not finite", (long long)t);
+    if (__builtin_popcountll(xmask[t]) > T)
+      return fail(QB_ERR_UNSUPPORTED, "rotation %lld has X / Y on %d qubits; at most %d fit the rotation tile", (long long)t,
+                  __builtin_popcountll(xmask[t]), T);
+  }
+  Guard g(s->ctx);
+  QB_TRY(check_state(s));
+  auto logical = [n](uint64_t m) {  // reference qubit q is logical bit n - 1 - q
+    uint64_t r = 0;
+    for (; m; m &= m - 1) r |= 1ull << (n - 1 - __builtin_ctzll(m));
+    return r;
+  };
+  for (int64_t t = 0; t < nrot; ++t) {
+    LogOp o;
+    o.kind = LOG_PAULI;
+    o.ctrl = logical(xmask[t]);
+    o.pz = logical(zmask[t]);
+    o.m[0] = std::cos(0.5 * theta[t]);
+    o.m[1] = std::sin(0.5 * theta[t]);
+    QB_TRY(append(s, std::move(o)));
   }
   return QB_OK;
 }

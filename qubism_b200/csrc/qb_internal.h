@@ -179,7 +179,7 @@ inline uint32_t swz_host(uint32_t u) {
 
 // ------------------------------------------------------------------ host-side ops
 struct HostOp {
-  int kind = 0;             // 0 = (controlled) 1q, 2 = dense kq (barrier op)
+  int kind = 0;             // 0 = (controlled) 1q, 2 = dense kq (barrier op), 3 = Pauli rotation (barrier op)
   uint32_t type = G_GENERAL;
   int target = -1;          // LOGICAL bit position (n-1-q)
   uint64_t ctrl = 0;        // mask over LOGICAL bit positions
@@ -188,6 +188,8 @@ struct HostOp {
   int k = 0;
   int kq_bits[QB_MAX_KQ] = {0};  // logical bit positions, kq_bits[0] = most significant index bit
   std::vector<double> kq_m;
+  // Pauli rotation cos(theta/2) I - i sin(theta/2) P: X / Z masks over LOGICAL bit positions; (c, s) in m[0], m[1]
+  uint64_t px = 0, pz = 0;
   // peephole bookkeeping
   bool dead = false;
   int nprev = 0;
@@ -317,6 +319,8 @@ std::string describe_plan(const PlanResult &r);
 //   - an uncontrolled 1q gate directly following another on the same qubit is merged into it
 //     (2x2 product on the host);
 //   - a controlled-X directly following the identical controlled-X cancels (cx . cx = I).
+// Dense blocks and Pauli rotations are never merged or cancelled; the identity Pauli string is a
+// global factor whatever the peephole setting.
 struct OpQueue {
   int n = 0;
   bool peephole = true;
@@ -332,6 +336,7 @@ struct OpQueue {
   void mul_gscale(double re, double im);
   void push_1q(int target_bit, uint64_t ctrl_mask, const double m[8]);
   void push_kq(const int *bits, int k, const double *m, uint64_t ctrl_mask);
+  void push_pauli(uint64_t xmask, uint64_t zmask, double c, double s);  // logical masks, c = cos(theta/2), s = sin
 };
 
 // ------------------------------------------------------------------ multi-GPU host logic

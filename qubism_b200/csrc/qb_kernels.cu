@@ -1210,6 +1210,111 @@ cudaError_t launch_expect_pauli(const double2 *amps, int local_bits, const ExpTe
   return expect_launch<64>(amps, npairs, terms, partials_dev, out_dev, sm_count, stream);
 }
 
+// ---------------------------------------------------------------- Pauli rotations
+// exp(-i theta/2 P) = c I - i s P pairs every amplitude j with exactly one partner j ^ x, so a rotation of
+// any weight is one 2x2 update per pair; a CTA that holds every X bit of a run of rotations in its tile
+// applies the whole run between one load and one store of that tile.  The tile goes straight from global
+// to XOR-swizzled shared memory (cp.async: no register staging), thread t owning tile-local indices
+// t + k * kPauliThreads (8 consecutive lanes = one 128-byte line while the low physical bits are tile
+// bits).  Consecutive Z-only rotations are one step: a phase per amplitude over the thread's own indices,
+// applied in one read and write of each.  A rotation with X is one step of one pair per thread and
+// iteration (swz keeps the partners conflict-free, being linear over XOR).  A CTA barrier separates two
+// steps unless both are Z-only steps; the store reads the thread's own indices again.
+__device__ __forceinline__ void pauli_phases(double2 &v, const PauliRotParam &p, uint32_t u, uint32_t sgn0) {
+  const bool neg = (__popc(u & p.zt) ^ sgn0) & 1u;
+  const double fr = neg ? p.c - p.ar : p.c + p.ar, fi = neg ? -p.ai : p.ai;
+  v = make_double2(fr * v.x - fi * v.y, fr * v.y + fi * v.x);
+}
+
+template <int TB>
+__global__ void __launch_bounds__(kPauliThreads, 3) k_pauli_rot_tile(double2 *__restrict__ amps, const __grid_constant__ PauliRotArgs a) {
+  constexpr int kThrBits = 8;
+  static_assert(kPauliThreads == 1 << kThrBits && TB > kThrBits, "tile-local index = thread + k * kPauliThreads");
+  constexpr int EPT = 1 << (TB - kThrBits);  // amplitudes per thread
+  extern __shared__ double2 tile[];
+  const uint32_t tid = threadIdx.x, tb = a.tile_bits, nel = 1u << tb, nrot = a.nrot;
+  uint64_t base = 0;  // the block number deposited into the local bits outside the tile
+  {
+    uint64_t t = blockIdx.x;
+    for (uint32_t i = 0; i < a.nruns; ++i) {
+      base |= (t & ((1ull << a.run_len[i]) - 1ull)) << a.run_shift[i];
+      t >>= a.run_len[i];
+    }
+  }
+  uint64_t off_lo = base, off_hi[TB - kThrBits];
+#pragma unroll
+  for (int b = 0; b < kThrBits; ++b)
+    if (b < (int)tb && ((tid >> b) & 1u)) off_lo |= 1ull << a.tile_pos[b];
+#pragma unroll
+  for (int b = 0; b < TB - kThrBits; ++b) off_hi[b] = b + kThrBits < (int)tb ? 1ull << a.tile_pos[b + kThrBits] : 0ull;
+  auto goff = [&](int k) {
+    uint64_t o = off_lo;
+#pragma unroll
+    for (int b = 0; b < TB - kThrBits; ++b)
+      if ((k >> b) & 1) o |= off_hi[b];
+    return o;
+  };
+  auto sign0 = [&](const PauliRotParam &p) { return uint32_t(__popcll(base & p.zout)) & 1u; };
+#pragma unroll
+  for (int k = 0; k < EPT; ++k)
+    if (tid + k * kPauliThreads < nel) {
+      const uint32_t sa = uint32_t(__cvta_generic_to_shared(tile + swz(tid + k * kPauliThreads)));
+      asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(amps + goff(k)) : "memory");
+    }
+  asm volatile("cp.async.wait_all;" ::: "memory");  // (own indices: visible to this thread, no barrier)
+  bool own = true;  // the last step wrote the thread's own indices only
+  for (uint32_t r = 0; r < nrot;) {
+    const PauliRotParam &p = a.rot[r];
+    if (p.xt == 0) {  // Z-only rotations r .. e
+      uint32_t e = r + 1;
+      while (e < nrot && a.rot[e].xt == 0) ++e;
+      if (!own) __syncthreads();
+#pragma unroll 4
+      for (int k = 0; k < EPT; ++k) {
+        const uint32_t u = tid + k * kPauliThreads;
+        if (u >= nel) continue;
+        double2 v = tile[swz(u)];
+        for (uint32_t z = r; z < e; ++z) pauli_phases(v, a.rot[z], u, sign0(a.rot[z]));
+        tile[swz(u)] = v;
+      }
+      own = true;
+      r = e;
+      continue;
+    }
+    __syncthreads();
+    const uint32_t h = 31 - __clz(p.xt), lo = (1u << h) - 1u, s0 = sign0(p);  // pairs (j, j ^ xt), bit h of j clear
+#pragma unroll 4
+    for (int k = 0; k < EPT / 2; ++k) {
+      const uint32_t q = tid + k * kPauliThreads;
+      if (q >= nel / 2) continue;
+      const uint32_t j = ((q & ~lo) << 1) | (q & lo), jx = j ^ p.xt;
+      const double2 A = tile[swz(j)], B = tile[swz(jx)];
+      const bool nj = (__popc(j & p.zt) ^ s0) & 1u, nk = (__popc(jx & p.zt) ^ s0) & 1u;
+      const double br = nk ? -B.x : B.x, bi = nk ? -B.y : B.y, ar = nj ? -A.x : A.x, ai = nj ? -A.y : A.y;
+      tile[swz(j)] = make_double2(p.c * A.x + p.ar * br - p.ai * bi, p.c * A.y + p.ar * bi + p.ai * br);
+      tile[swz(jx)] = make_double2(p.c * B.x + p.ar * ar - p.ai * ai, p.c * B.y + p.ar * ai + p.ai * ar);
+    }
+    own = false;
+    ++r;
+  }
+  if (!own) __syncthreads();
+#pragma unroll
+  for (int k = 0; k < EPT; ++k)
+    if (tid + k * kPauliThreads < nel) __stcs(amps + goff(k), tile[swz(tid + k * kPauliThreads)]);
+}
+
+cudaError_t launch_pauli_rot(double2 *amps, int local_bits, const PauliRotArgs &args, cudaStream_t stream) {
+  if (args.nrot < 1 || args.nrot > (uint32_t)kPauliMaxRot || args.tile_bits > (uint32_t)kPauliTileBits ||
+      (int)args.tile_bits > local_bits)
+    return cudaErrorInvalidValue;
+  const size_t smem = sizeof(double2) << args.tile_bits;
+  const auto fn = k_pauli_rot_tile<kPauliTileBits>;
+  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, int(sizeof(double2) << kPauliTileBits));
+  if (e != cudaSuccess) return e;
+  fn<<<unsigned(1ull << (local_bits - args.tile_bits)), kPauliThreads, smem, stream>>>(amps, args);
+  return cudaGetLastError();
+}
+
 // ---------------------------------------------------------------- live sub-cube kernels
 // After a collapse (StateVec.hs:104-114) half of the state is exactly zero, and a fresh
 // |0...0> is zero outside one amplitude.  The host tracks the index bits whose value is KNOWN

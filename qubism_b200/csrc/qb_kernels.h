@@ -55,6 +55,28 @@ struct ExpTerms {
 cudaError_t launch_expect_pauli(const double2 *amps, int local_bits, const ExpTerms &terms, double *partials_dev,
                                 double *out_dev, int sm_count, cudaStream_t stream);
 
+// Pauli rotations exp(-i theta/2 P) in place (qb_apply_pauli_rot): up to kPauliMaxRot rotations in ONE
+// read + write sweep.  A CTA owns a tile of 2^tile_bits amplitudes on the physical bits tile_pos[] (every X
+// bit of the launch is one of them); rotation r, for every tile-local index j, sets
+//   psi'_j = c psi_j + (ar + i ai) (-1)^popc((j ^ xt) & zt) (-1)^popc(base & zout) psi_(j ^ xt)
+// with base = the tile's non-tile bits.  The host folds -i sin(theta/2) i^popc(x & z) and the sign of Z on
+// global qubits into (ar, ai).  xt == 0 (Z only) is a per-amplitude phase.
+constexpr int kPauliTileBits = 12;  // 64 KB of shared memory per CTA
+constexpr int kPauliMaxRot = 64;
+constexpr int kPauliThreads = 256;
+struct PauliRotParam {
+  uint64_t zout;       // Z mask on the local bits outside the tile (physical)
+  double c, ar, ai;    // cos(theta/2); the partner's factor
+  uint32_t xt, zt;     // X / Z masks on the tile-local bits
+};
+struct PauliRotArgs {
+  uint32_t nrot, tile_bits, nruns, _pad;
+  uint8_t tile_pos[16];                 // physical bit of tile-local bit i, ascending
+  uint8_t run_shift[16], run_len[16];   // the tile number deposited into the local bits outside the tile
+  PauliRotParam rot[kPauliMaxRot];
+};
+cudaError_t launch_pauli_rot(double2 *amps, int local_bits, const PauliRotArgs &args, cudaStream_t stream);
+
 // Live sub-cube {i : i & fixed_mask == fixed_val} of the shard (see "support" in qb_api.cpp): the
 // reduction of launch_sumsq restricted to it, and zero-fill (mode 0) / scaling (mode 1) of it.
 int cube_runs(int local_bits, uint64_t fixed_mask);  // must be <= kMaxRuns for the launchers below

@@ -434,6 +434,25 @@ void OpQueue::push_kq(const int *bits, int k, const double *m, uint64_t ctrl_mas
   ops.push_back(std::move(op));
 }
 
+void OpQueue::push_pauli(uint64_t xmask, uint64_t zmask, double c, double s) {
+  ++submitted;
+  if (!(xmask | zmask)) {  // exp(-i theta/2 I): a global factor
+    mul_gscale(c, -s);
+    ++folded;
+    return;
+  }
+  HostOp op;
+  op.kind = 3;
+  op.px = xmask;
+  op.pz = zmask;
+  op.m[0] = c;
+  op.m[1] = s;
+  const int idx = (int)ops.size();
+  link_op(*this, op, idx, xmask | zmask);
+  op.nprev = 7;  // never merged / cancelled
+  ops.push_back(std::move(op));
+}
+
 // --------------------------------------------------------------------- multi-GPU swap logic
 std::vector<SwapPair> choose_swaps(int n, int L, const std::vector<int> &perm,
                                    const std::vector<const HostOp *> &pending, bool any_local,
@@ -447,6 +466,16 @@ std::vector<SwapPair> choose_swaps(int n, int L, const std::vector<int> &perm,
     if (h.kind == 2) {  // a dense block runs unfused and needs ALL its qubits inside the shard
       for (int j = 0; j < h.k; ++j) {
         const int pb = perm[h.kq_bits[j]];
+        if (pb >= L && !(seen & (1ull << pb))) {
+          seen |= 1ull << pb;
+          need.push_back(pb);
+        }
+      }
+      continue;
+    }
+    if (h.kind == 3) {  // a Pauli rotation pairs amplitudes across its X qubits: those must be inside the shard
+      for (uint64_t m = h.px; m; m &= m - 1) {
+        const int pb = perm[__builtin_ctzll(m)];
         if (pb >= L && !(seen & (1ull << pb))) {
           seen |= 1ull << pb;
           need.push_back(pb);
@@ -482,6 +511,7 @@ std::vector<SwapPair> choose_swaps(int n, int L, const std::vector<int> &perm,
         if (h.kind == 2)
           for (int j = 0; j < h.k; ++j)
             if (h.kq_bits[j] == logical_of[b]) next = std::min(next, (long)i);
+        if (h.kind == 3 && ((h.px >> logical_of[b]) & 1ull)) next = std::min(next, (long)i);
       }
       // not needed again in this flush: if the caller knows what comes after it (the same op
       // stream again, for an iterated circuit), look there -- the qubits that end a step on the

@@ -314,6 +314,18 @@ class StateVec:
                                               out.ctypes.data_as(C.POINTER(C.c_double))))
         return out
 
+    def pauli_rot_(self, terms, thetas):
+        """Apply ``exp(-i theta/2 P)`` for each Pauli string ``P`` of ``terms`` with the angle of ``thetas``, in
+        order, in place (qb_apply_pauli_rot).  Terms are spelled as for ``expect_pauli``.  Queued like a gate."""
+        xs, zs = pauli_masks(terms, self.n)
+        th = np.ascontiguousarray(thetas, dtype=np.float64).reshape(-1)
+        if th.size != xs.size:
+            raise ValueError(f"{xs.size} Pauli strings but {th.size} angles")
+        P64 = C.POINTER(C.c_uint64)
+        capi.check(self.ctx.L.qb_apply_pauli_rot(self._h, xs.ctypes.data_as(P64), zs.ctypes.data_as(P64),
+                                                 th.ctypes.data_as(C.POINTER(C.c_double)), len(xs)))
+        return self
+
     def norm(self) -> float:  # Algebra.hs:35-36: realPart (a <.> a), the SQUARED norm
         return self.inner(self).real
 
@@ -395,3 +407,9 @@ def measure(sv: StateVec, rs) -> list:
 def expectPauli(terms, sv: StateVec) -> np.ndarray:
     """``[realPart (sv <.> (p #> sv)) | p <- terms]`` without building any ``p #> sv`` (see StateVec.expect_pauli)."""
     return sv.expect_pauli(terms)
+
+
+def pauliRotate(terms, thetas, sv: StateVec) -> StateVec:
+    """``exp(-i theta_k/2 P_k) ... exp(-i theta_0/2 P_0) #> sv`` as a new value; ``sv`` keeps its own
+    (a lazy clone rotated in place, see StateVec.pauli_rot_)."""
+    return sv.clone().pauli_rot_(terms, thetas)
