@@ -56,3 +56,6 @@ foreign import ccall safe   "qb_tensor"          c_qb_tensor          :: Ptr QbS
 foreign import ccall safe   "qb_expect_pauli"    c_qb_expect_pauli    :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Int64 -> Ptr CDouble -> IO CInt
 -- Pauli rotations ------------------------------------------------------------------------
 foreign import ccall safe   "qb_apply_pauli_rot" c_qb_apply_pauli_rot :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Ptr CDouble -> Int64 -> IO CInt
+-- Pauli sums and adjoint gradients ------------------------------------------------------------
+foreign import ccall safe   "qb_pauli_sum"       c_qb_pauli_sum       :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Ptr C -> Int64 -> Ptr (Ptr QbState) -> IO CInt
+foreign import ccall safe   "qb_pauli_rot_grad"  c_qb_pauli_rot_grad  :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Ptr CDouble -> Int64 -> Ptr Word64 -> Ptr Word64 -> Ptr CDouble -> Int64 -> Ptr CDouble -> Ptr CDouble -> IO CInt

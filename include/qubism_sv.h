@@ -215,6 +215,38 @@ int qb_expect_pauli(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, i
 #define QB_PAULI_ROT_MAX_X 12
 int qb_apply_pauli_rot(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, const double *theta, int64_t nrot);
 
+/* ---- Pauli sums and adjoint gradients --------------------------------------------------- */
+/* *out = (sum_t coef[t] P_t) #> src as a NEW state; src keeps its value.  Strings as in
+ * qb_expect_pauli; coef: nterms complex numbers.  Duplicate strings add; an empty sum gives the zero
+ * vector.  Observes src (flushes it).  Distributed: a collective.
+ * Cost: one read of src and one write of *out per run of terms whose X qubits fit one tile of
+ * QB_PAULI_ROT_MAX_X qubits together, at most 64 terms each, after grouping the terms by X mask (later
+ * runs also read *out); counted in qb_stats.simple_launches.  Sharded: X / Y on global qubits first swap
+ * those qubits into src's shard, and *out follows src's layout.  *out knows the qubits of known value
+ * (|0...0>, after a collapse) that src knows outside every term's X mask.
+ *
+ * Adjoint gradient of a Pauli-sum energy over a list of Pauli rotations:
+ *   psi     = R_{P_{K-1}}(theta[K-1]) ... R_{P_0}(theta[0]) s   (what qb_apply_pauli_rot would make)
+ *   *energy = sum_t hcoef[t] * realPart (psi <.> (H_t #> psi))  (real hcoef: H is Hermitian; not normalised)
+ *   grad[k] = d(*energy) / d(theta[k])                           (0 for the identity string)
+ * s keeps its value and its handle (also with option "linear" = 1).  Deterministic.  Distributed: a
+ * collective; every rank passes the same arguments and receives the same energy and gradient.
+ * Cost: a copy of s and the forward rotations (as qb_apply_pauli_rot), one H psi as qb_pauli_sum that also
+ * yields the energy, and one backward sweep per launch of the rotations' cut, reading and writing two
+ * states (simple_launches; one reduce_launches each for every sum and backward launch).  Memory: two
+ * temporary states.
+ * Both calls check everything before anything is queued or allocated (a rejected call leaves the
+ * state and its queue untouched):
+ * QB_ERR_ARG: a null pointer with a count > 0, a negative count, a mask bit at or above n, a
+ * non-finite theta or coefficient.  QB_ERR_UNSUPPORTED: a rotation string or a term of H with X / Y on
+ * more than QB_PAULI_ROT_MAX_X qubits, or on more qubits than a shard holds.  QB_ERR_OOM: no room for
+ * the temporary states (s / src stays valid). */
+int qb_pauli_sum(qb_state *src, const uint64_t *xmask, const uint64_t *zmask, const qb_c64 *coef, int64_t nterms,
+                 qb_state **out);
+int qb_pauli_rot_grad(qb_state *s, const uint64_t *rx, const uint64_t *rz, const double *theta, int64_t nrot,
+                      const uint64_t *hx, const uint64_t *hz, const double *hcoef, int64_t nterms, double *energy,
+                      double *grad);
+
 /* ---- introspection (tests, bench, profiling) ------------------------------------------- */
 typedef struct {
   uint64_t ops_submitted;   /* primitive ops received through the ABI                     */

@@ -92,6 +92,9 @@ SIGNATURES = {
     "qb_tensor": (_I, [_VP, _VP, C.POINTER(_VP)]),
     "qb_expect_pauli": (_I, [_VP, C.POINTER(_U64), C.POINTER(_U64), _I64, C.POINTER(_D)]),
     "qb_apply_pauli_rot": (_I, [_VP, C.POINTER(_U64), C.POINTER(_U64), C.POINTER(_D), _I64]),
+    "qb_pauli_sum": (_I, [_VP, C.POINTER(_U64), C.POINTER(_U64), _VP, _I64, C.POINTER(_VP)]),
+    "qb_pauli_rot_grad": (_I, [_VP, C.POINTER(_U64), C.POINTER(_U64), C.POINTER(_D), _I64, C.POINTER(_U64),
+                               C.POINTER(_U64), C.POINTER(_D), _I64, C.POINTER(_D), C.POINTER(_D)]),
     "qb_get_stats": (_I, [_VP, C.POINTER(QbStats)]),
     "qb_reset_stats": (_I, [_VP]),
     "qb_ctx_stream": (_VP, [_VP]),

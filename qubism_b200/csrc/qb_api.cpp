@@ -867,53 +867,80 @@ void support_after_op(Buffer *s, const HostOp &op) {
   s->zval &= s->zmask;
 }
 
-// A stretch of consecutive Pauli rotations (HostOp kind 3), cut greedily into launches of k_pauli_rot_tile
-// (one read + write sweep each).  A rotation joins the running launch while that holds fewer than
-// kPauliMaxRot and its X qubits add nothing to the launch's X union or the union with the three low
-// physical bits (one 128-byte line) still fits the tile; the tile is that union topped up with the lowest
-// other local bits.  Sharded: the launch's X qubits are brought into the shard first, and Z on global qubits
-// becomes this rank's sign.
+// The greedy launch cut of the Pauli kernels (k_pauli_rot_tile, k_pauli_sum_tile, k_pauli_rot_adjoint_tile):
+// the launch that starts at string i0 of lx (logical X masks) ends before the returned index.  A string joins
+// the running launch while that holds fewer than kPauliMaxRot and its X qubits add nothing to the launch's X
+// union or the union with the three low physical bits (one 128-byte line) still fits the tile.  *ux = the
+// launch's logical X union.
 static_assert(kPauliTileBits == QB_PAULI_ROT_MAX_X, "the tile holds the widest string the header allows");
+size_t pauli_cut(const Buffer *s, const std::vector<uint64_t> &lx, size_t i0, uint64_t *ux) {
+  const int T = std::min(kPauliTileBits, s->L);
+  const uint64_t low = (1ull << std::min(3, s->L)) - 1ull;
+  *ux = 0;
+  size_t i1 = i0;
+  for (; i1 < lx.size() && i1 - i0 < size_t(kPauliMaxRot); ++i1) {
+    const uint64_t x = lx[i1];
+    if (i1 > i0 && (x & ~*ux) && __builtin_popcountll(phys_mask(s, *ux | x) | low) > T) break;
+    *ux |= x;
+  }
+  return i1;
+}
+
+// The tile of a launch whose logical X union is ux (already inside the shard): those physical bits topped up
+// with the lowest other local bits.  Fills the tile geometry shared by the Pauli kernels' argument blocks.
+template <class A>
+int pauli_tile(const Buffer *s, uint64_t ux, A &args) {
+  const int L = s->L, T = std::min(kPauliTileBits, L);
+  uint64_t tile = phys_mask(s, ux);
+  if (__builtin_popcountll(tile) > T || (tile >> L))
+    return fail(QB_ERR_UNSUPPORTED, "internal: Pauli strings with X outside the rotation tile");
+  for (int b = 0; __builtin_popcountll(tile) < T; ++b) tile |= 1ull << b;
+  args.tile_bits = uint32_t(T);
+  for (int b = 0, i = 0; b < L; ++b)
+    if ((tile >> b) & 1ull) args.tile_pos[i++] = uint8_t(b);
+  for (int b = 0; b < L;) {  // runs of the local bits outside the tile
+    if ((tile >> b) & 1ull) {
+      ++b;
+      continue;
+    }
+    int e = b;
+    while (e < L && !((tile >> e) & 1ull)) ++e;
+    args.run_shift[args.nruns] = uint8_t(b);
+    args.run_len[args.nruns++] = uint8_t(e - b);
+    b = e;
+  }
+  return QB_OK;
+}
+
+// a physical mask on the tile-local bits of a launch
+template <class A>
+uint32_t pauli_tile_local(const A &args, uint64_t m) {
+  uint32_t r = 0;
+  for (uint32_t i = 0; i < args.tile_bits; ++i) r |= uint32_t((m >> args.tile_pos[i]) & 1ull) << i;
+  return r;
+}
+
+// A stretch of consecutive Pauli rotations (HostOp kind 3), cut by pauli_cut into launches of
+// k_pauli_rot_tile (one read + write sweep each).  Sharded: the launch's X qubits are brought into the shard
+// first, and Z on global qubits becomes this rank's sign.
 int run_pauli_rots(Buffer *s, const std::vector<const HostOp *> &run) {
   qb_ctx *c = s->ctx;
   QB_TRY(ensure_inplace(s));
-  const int L = s->L, T = std::min(kPauliTileBits, L);
-  const uint64_t local = (1ull << L) - 1ull, low = (1ull << std::min(3, L)) - 1ull;
+  const int L = s->L;
+  const uint64_t local = (1ull << L) - 1ull;
+  std::vector<uint64_t> lx;
+  for (const HostOp *h : run) lx.push_back(h->px);
   for (size_t i0 = 0; i0 < run.size();) {
     uint64_t ux = 0;  // logical X union of the launch
-    size_t i1 = i0;
-    for (; i1 < run.size() && i1 - i0 < size_t(kPauliMaxRot); ++i1) {
-      const uint64_t x = run[i1]->px;
-      if (i1 > i0 && (x & ~ux) && __builtin_popcountll(phys_mask(s, ux | x) | low) > T) break;
-      ux |= x;
-    }
+    const size_t i1 = pauli_cut(s, lx, i0, &ux);
     if (c->nranks > 1) QB_TRY(localise_x(s, ux));
-    uint64_t tile = phys_mask(s, ux);
-    if (__builtin_popcountll(tile) > T || (tile & ~local))
-      return fail(QB_ERR_UNSUPPORTED, "internal: Pauli rotations with X outside the rotation tile");
-    for (int b = 0; __builtin_popcountll(tile) < T; ++b) tile |= 1ull << b;
     PauliRotArgs args;
     memset(&args, 0, sizeof args);
     args.nrot = uint32_t(i1 - i0);
-    args.tile_bits = uint32_t(T);
-    for (int b = 0, i = 0; b < L; ++b)
-      if ((tile >> b) & 1ull) args.tile_pos[i++] = uint8_t(b);
-    for (int b = 0; b < L;) {  // runs of the local bits outside the tile
-      if ((tile >> b) & 1ull) {
-        ++b;
-        continue;
-      }
-      int e = b;
-      while (e < L && !((tile >> e) & 1ull)) ++e;
-      args.run_shift[args.nruns] = uint8_t(b);
-      args.run_len[args.nruns++] = uint8_t(e - b);
-      b = e;
-    }
-    auto tile_local = [&](uint64_t m) {
-      uint32_t r = 0;
-      for (int i = 0; i < T; ++i) r |= uint32_t((m >> args.tile_pos[i]) & 1ull) << i;
-      return r;
-    };
+    QB_TRY(pauli_tile(s, ux, args));
+    uint64_t tile = 0;
+    for (uint32_t i = 0; i < args.tile_bits; ++i) tile |= 1ull << args.tile_pos[i];
+    auto tile_local = [&](uint64_t m) { return pauli_tile_local(args, m); };
     for (size_t i = i0; i < i1; ++i) {
       const HostOp &h = *run[i];
       const uint64_t xp = phys_mask(s, h.px), zp = phys_mask(s, h.pz);
@@ -1392,6 +1419,119 @@ void drop_handle(qb_state *s) {
   }
   delete s;
   if (last_of_closed) delete c;
+}
+
+// reference qubit q is logical bit n - 1 - q
+uint64_t logical_mask(int n, uint64_t m) {
+  uint64_t r = 0;
+  for (; m; m &= m - 1) r |= 1ull << (n - 1 - __builtin_ctzll(m));
+  return r;
+}
+
+// (re, im) * i^popc(x & z) * this rank's sign of Z on global qubits: the factor of P = i^ph X^x Z^z that the
+// tile kernels do not form (Y = i X Z)
+void pauli_phase(const Buffer *s, uint64_t lx, uint64_t lz, double re, double im, double *out_re, double *out_im) {
+  if (__builtin_popcountll((phys_mask(s, lz) >> s->L) & uint64_t(s->ctx->rank)) & 1) {
+    re = -re;
+    im = -im;
+  }
+  switch (__builtin_popcountll(lx & lz) & 3) {
+    case 0: *out_re = re; *out_im = im; break;
+    case 1: *out_re = -im; *out_im = re; break;
+    case 2: *out_re = -re; *out_im = -im; break;
+    default: *out_re = im; *out_im = -re; break;
+  }
+}
+
+// out <- (sum_t coef[t] P_t) src, P_t named by logical masks; out is a fresh shard of src's size whose old
+// contents do not matter.  Terms are taken in the order of their X masks (a sum commutes; a stable sort, so
+// the order is a fixed function of the input) and cut by pauli_cut.  The first launch writes every amplitude
+// of out in src's layout; later launches add, out following src's layout (localise_x) by relayout.
+// energy_dev: Re <src| H_launch src> of launch l into energy_dev[l], *nlaunch = the number of launches.
+int run_pauli_sum(Buffer *src, Buffer *out, const std::vector<uint64_t> &lx, const std::vector<uint64_t> &lz,
+                  const std::vector<double> &coef, double *energy_dev, int *nlaunch) {
+  qb_ctx *c = src->ctx;
+  QB_TRY(ensure_inplace(src));
+  const uint64_t local = (1ull << src->L) - 1ull;
+  std::vector<size_t> ord(lx.size());
+  for (size_t t = 0; t < ord.size(); ++t) ord[t] = t;
+  std::stable_sort(ord.begin(), ord.end(), [&](size_t a, size_t b) { return lx[a] < lx[b]; });
+  std::vector<uint64_t> sx(ord.size());
+  for (size_t t = 0; t < ord.size(); ++t) sx[t] = lx[ord[t]];
+  int nl = 0;
+  for (size_t i0 = 0; i0 < sx.size(); ++nl) {
+    uint64_t ux = 0;
+    const size_t i1 = pauli_cut(src, sx, i0, &ux);
+    if (c->nranks > 1) QB_TRY(localise_x(src, ux));
+    if (nl == 0) out->perm = src->perm;  // (the first launch writes every amplitude: born in src's layout)
+    else if (out->perm != src->perm) QB_TRY(relayout(out, src->perm));
+    PauliSumArgs args;
+    memset(&args, 0, sizeof args);
+    args.nterms = uint32_t(i1 - i0);
+    args.first = nl == 0;
+    QB_TRY(pauli_tile(src, ux, args));
+    uint64_t tile = 0;
+    for (uint32_t i = 0; i < args.tile_bits; ++i) tile |= 1ull << args.tile_pos[i];
+    for (size_t i = i0; i < i1; ++i) {
+      const size_t t = ord[i];
+      const uint64_t zp = phys_mask(src, lz[t]);
+      PauliSumParam &p = args.term[i - i0];
+      p.xt = pauli_tile_local(args, phys_mask(src, lx[t]));
+      p.zt = pauli_tile_local(args, zp);
+      p.zout = zp & local & ~tile;
+      pauli_phase(src, lx[t], lz[t], coef[2 * t], coef[2 * t + 1], &p.cr, &p.ci);
+    }
+    QB_CUDA(launch_pauli_sum(src->amps, out->amps, src->L, args, energy_dev ? c->red_partials : nullptr,
+                             energy_dev ? energy_dev + nl : nullptr, c->sm_count, c->stream));
+    c->stats.simple_launches++;
+    if (energy_dev) c->stats.reduce_launches++;
+    i0 = i1;
+  }
+  if (nlaunch) *nlaunch = nl;
+  return QB_OK;
+}
+
+// The backward pass of the adjoint gradient: psi = the state after the rotations (lx, lz, cos / sin of
+// theta / 2 in cs, none the identity), lam = H psi in the same layout.  The cut of pauli_cut is walked from its
+// last launch to its first, each launch's rotations from last to first; grad_dev[k] = Im <lam_{k+1}| P_k
+// |psi_{k+1}> of rotation k.  psi and lam end with every rotation undone.
+int run_pauli_adjoint(Buffer *psi, Buffer *lam, const std::vector<uint64_t> &lx, const std::vector<uint64_t> &lz,
+                      const std::vector<double> &cs, double *grad_dev) {
+  qb_ctx *c = psi->ctx;
+  const uint64_t local = (1ull << psi->L) - 1ull;
+  std::vector<std::pair<size_t, uint64_t>> cut;  // (first rotation, X union) of each launch
+  for (size_t i0 = 0; i0 < lx.size();) {
+    uint64_t ux = 0;
+    const size_t i1 = pauli_cut(psi, lx, i0, &ux);
+    cut.emplace_back(i0, ux);
+    i0 = i1;
+  }
+  for (size_t l = cut.size(); l-- > 0;) {
+    const size_t i0 = cut[l].first, i1 = l + 1 < cut.size() ? cut[l + 1].first : lx.size();
+    if (c->nranks > 1) QB_TRY(localise_x(psi, cut[l].second));
+    if (lam->perm != psi->perm) QB_TRY(relayout(lam, psi->perm));
+    PauliAdjArgs args;
+    memset(&args, 0, sizeof args);
+    args.nrot = uint32_t(i1 - i0);
+    QB_TRY(pauli_tile(psi, cut[l].second, args));
+    uint64_t tile = 0;
+    for (uint32_t i = 0; i < args.tile_bits; ++i) tile |= 1ull << args.tile_pos[i];
+    for (size_t k = i0; k < i1; ++k) {
+      const uint64_t zp = phys_mask(psi, lz[k]);
+      PauliAdjParam &p = args.rot[k - i0];
+      p.xt = pauli_tile_local(args, phys_mask(psi, lx[k]));
+      p.zt = pauli_tile_local(args, zp);
+      p.zout = zp & local & ~tile;
+      p.c = cs[2 * k];
+      p.s = cs[2 * k + 1];
+      pauli_phase(psi, lx[k], lz[k], 1.0, 0.0, &p.fr, &p.fi);
+    }
+    QB_CUDA(launch_pauli_rot_adjoint(psi->amps, lam->amps, psi->L, args, c->red_partials, grad_dev + i0, c->sm_count,
+                                     c->stream));
+    c->stats.simple_launches++;
+    c->stats.reduce_launches++;
+  }
+  return QB_OK;
 }
 
 }  // namespace
@@ -2057,36 +2197,173 @@ int qb_expect_pauli(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, i
 }
 
 // ---- Pauli rotations
-int qb_apply_pauli_rot(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, const double *theta, int64_t nrot) {
-  if (!s) return fail(QB_ERR_ARG, "null state");
-  if (nrot < 0) return fail(QB_ERR_ARG, "nrot %lld < 0", (long long)nrot);
-  if (nrot == 0) return QB_OK;
-  if (!xmask || !zmask || !theta) return fail(QB_ERR_ARG, "null argument");
+// The checks of count strings for the tile kernels, made before anything is queued or allocated: the masks
+// name qubits of s, the values v[t * nv .. t * nv + nv) are finite, and X / Y fit the rotation tile.
+static int check_pauli_strings(const qb_state *s, const char *what, const char *value, const uint64_t *xmask,
+                               const uint64_t *zmask, const double *v, int nv, int64_t count) {
   const int n = s->n, T = std::min(kPauliTileBits, s->n - s->ctx->pbits);
-  for (int64_t t = 0; t < nrot; ++t) {  // everything is checked before anything is queued
-    if ((xmask[t] | zmask[t]) >> n) return fail(QB_ERR_ARG, "rotation %lld names a qubit >= %d", (long long)t, n);
-    if (!std::isfinite(theta[t])) return fail(QB_ERR_ARG, "rotation %lld: theta is not finite", (long long)t);
+  for (int64_t t = 0; t < count; ++t) {
+    if ((xmask[t] | zmask[t]) >> n) return fail(QB_ERR_ARG, "%s %lld names a qubit >= %d", what, (long long)t, n);
+    for (int j = 0; j < nv; ++j)
+      if (!std::isfinite(v[t * nv + j])) return fail(QB_ERR_ARG, "%s %lld: %s is not finite", what, (long long)t, value);
     if (__builtin_popcountll(xmask[t]) > T)
-      return fail(QB_ERR_UNSUPPORTED, "rotation %lld has X / Y on %d qubits; at most %d fit the rotation tile", (long long)t,
-                  __builtin_popcountll(xmask[t]), T);
+      return fail(QB_ERR_UNSUPPORTED, "%s %lld has X / Y on %d qubits; at most %d fit the rotation tile", what,
+                  (long long)t, __builtin_popcountll(xmask[t]), T);
   }
-  Guard g(s->ctx);
-  QB_TRY(check_state(s));
-  auto logical = [n](uint64_t m) {  // reference qubit q is logical bit n - 1 - q
-    uint64_t r = 0;
-    for (; m; m &= m - 1) r |= 1ull << (n - 1 - __builtin_ctzll(m));
-    return r;
-  };
+  return QB_OK;
+}
+
+// append rotations (already checked) to s's lineage
+static int log_pauli_rots(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, const double *theta, int64_t nrot) {
   for (int64_t t = 0; t < nrot; ++t) {
     LogOp o;
     o.kind = LOG_PAULI;
-    o.ctrl = logical(xmask[t]);
-    o.pz = logical(zmask[t]);
+    o.ctrl = logical_mask(s->n, xmask[t]);
+    o.pz = logical_mask(s->n, zmask[t]);
     o.m[0] = std::cos(0.5 * theta[t]);
     o.m[1] = std::sin(0.5 * theta[t]);
     QB_TRY(append(s, std::move(o)));
   }
   return QB_OK;
+}
+
+int qb_apply_pauli_rot(qb_state *s, const uint64_t *xmask, const uint64_t *zmask, const double *theta, int64_t nrot) {
+  if (!s) return fail(QB_ERR_ARG, "null state");
+  if (nrot < 0) return fail(QB_ERR_ARG, "nrot %lld < 0", (long long)nrot);
+  if (nrot == 0) return QB_OK;
+  if (!xmask || !zmask || !theta) return fail(QB_ERR_ARG, "null argument");
+  QB_TRY(check_pauli_strings(s, "rotation", "theta", xmask, zmask, theta, 1, nrot));
+  Guard g(s->ctx);
+  QB_TRY(check_state(s));
+  return log_pauli_rots(s, xmask, zmask, theta, nrot);
+}
+
+// ---- Pauli sums
+int qb_pauli_sum(qb_state *src, const uint64_t *xmask, const uint64_t *zmask, const qb_c64 *coef, int64_t nterms,
+                 qb_state **out) {
+  if (!src || !out) return fail(QB_ERR_ARG, "null argument");
+  if (nterms < 0) return fail(QB_ERR_ARG, "nterms %lld < 0", (long long)nterms);
+  if (nterms > 0 && (!xmask || !zmask || !coef)) return fail(QB_ERR_ARG, "null argument");
+  static_assert(sizeof(qb_c64) == 2 * sizeof(double), "qb_c64 is (re, im)");
+  QB_TRY(check_pauli_strings(src, "term", "coefficient", xmask, zmask, reinterpret_cast<const double *>(coef), 2, nterms));
+  qb_ctx *c = src->ctx;
+  Guard g(c);
+  QB_TRY(materialise(src));
+  Buffer *b = src->b;
+  if (!(std::isfinite(b->pscale[0]) && std::isfinite(b->pscale[1]))) QB_TRY(force_scale(b));  // NaN / inf must reach the data
+  Buffer *ob = nullptr;
+  QB_TRY(new_buffer(c, src->n, &ob));
+  std::vector<uint64_t> lx(nterms), lz(nterms);
+  std::vector<double> cf(2 * nterms);
+  uint64_t xunion = 0;
+  for (int64_t t = 0; t < nterms; ++t) {
+    lx[t] = logical_mask(src->n, xmask[t]);
+    lz[t] = logical_mask(src->n, zmask[t]);
+    xunion |= lx[t];
+    cf[2 * t] = coef[t].re * b->pscale[0] - coef[t].im * b->pscale[1];  // the pending scalar rides on the coefficients
+    cf[2 * t + 1] = coef[t].re * b->pscale[1] + coef[t].im * b->pscale[0];
+  }
+  int rc = QB_OK;
+  if (nterms == 0) {
+    ob->perm = b->perm;
+    if (cudaMemsetAsync(ob->amps, 0, sizeof(double2) << ob->L, c->stream) != cudaSuccess) rc = fail(QB_ERR_CUDA, "zero fill");
+  } else {
+    rc = run_pauli_sum(b, ob, lx, lz, cf, nullptr, nullptr);
+  }
+  if (rc != QB_OK) {
+    release_buffer(ob);
+    return rc;
+  }
+  // P_t moves amplitude j to j ^ x_t: what the source knows outside every X mask still holds (§3.3b)
+  ob->all_finite = b->all_finite;
+  ob->zmask = ob->all_finite ? b->zmask & ~xunion : 0;
+  ob->zval = b->zval & ob->zmask;
+  return new_handle(c, ob, 0, out);
+}
+
+// ---- adjoint gradients of Pauli-sum energies
+int qb_pauli_rot_grad(qb_state *s, const uint64_t *rx, const uint64_t *rz, const double *theta, int64_t nrot,
+                      const uint64_t *hx, const uint64_t *hz, const double *hcoef, int64_t nterms, double *energy,
+                      double *grad) {
+  if (!s || !energy) return fail(QB_ERR_ARG, "null argument");
+  if (nrot < 0) return fail(QB_ERR_ARG, "nrot %lld < 0", (long long)nrot);
+  if (nterms < 0) return fail(QB_ERR_ARG, "nterms %lld < 0", (long long)nterms);
+  if (nrot > 0 && (!rx || !rz || !theta || !grad)) return fail(QB_ERR_ARG, "null argument");
+  if (nterms > 0 && (!hx || !hz || !hcoef)) return fail(QB_ERR_ARG, "null argument");
+  QB_TRY(check_pauli_strings(s, "rotation", "theta", rx, rz, theta, 1, nrot));
+  QB_TRY(check_pauli_strings(s, "term", "coefficient", hx, hz, hcoef, 1, nterms));
+  qb_ctx *c = s->ctx;
+  Guard g(c);
+  QB_TRY(check_state(s));
+  *energy = 0.0;
+  for (int64_t k = 0; k < nrot; ++k) grad[k] = 0.0;
+  if (nterms == 0) return QB_OK;  // H = 0
+  // psi: a copy of s that owns its shard (s keeps its value and its handle, also with option "linear")
+  qb_state *w = nullptr;
+  QB_TRY(qb_state_clone(s, &w));
+  Buffer *lam = nullptr;
+  double *dres = nullptr;
+  auto done = [&](int rc) {
+    if (dres) cudaFree(dres);
+    if (lam) release_buffer(lam);
+    drop_handle(w);
+    return rc;
+  };
+  int rc = split_off(w, false);
+  if (rc == QB_OK) rc = log_pauli_rots(w, rx, rz, theta, nrot);
+  if (rc == QB_OK) rc = materialise(w);
+  if (rc != QB_OK) return done(rc);
+  Buffer *psi = w->b;
+  if (!(std::isfinite(psi->pscale[0]) && std::isfinite(psi->pscale[1]))) {
+    if ((rc = force_scale(psi)) != QB_OK) return done(rc);
+  }
+  if ((rc = new_buffer(c, s->n, &lam)) != QB_OK) return done(rc);
+  // the rotations the backward pass walks: every one but the identity string (a global phase, gradient 0)
+  std::vector<int64_t> idx;
+  std::vector<uint64_t> lx, lz, hlx(nterms), hlz(nterms);
+  std::vector<double> cs, hc(2 * nterms);
+  for (int64_t k = 0; k < nrot; ++k)
+    if (rx[k] | rz[k]) {
+      idx.push_back(k);
+      lx.push_back(logical_mask(s->n, rx[k]));
+      lz.push_back(logical_mask(s->n, rz[k]));
+      cs.push_back(std::cos(0.5 * theta[k]));
+      cs.push_back(std::sin(0.5 * theta[k]));
+    }
+  for (int64_t t = 0; t < nterms; ++t) {
+    hlx[t] = logical_mask(s->n, hx[t]);
+    hlz[t] = logical_mask(s->n, hz[t]);
+    hc[2 * t] = hcoef[t];
+    hc[2 * t + 1] = 0.0;
+  }
+  const size_t nres = idx.size() + size_t(nterms);  // gradient of each walked rotation, energy of each sum launch
+  if (cudaMalloc(&dres, sizeof(double) * nres) != cudaSuccess) {
+    (void)cudaGetLastError();
+    dres = nullptr;
+    return done(fail(QB_ERR_OOM, "gradient scratch"));
+  }
+  int nl = 0;
+  if (cudaMemsetAsync(dres, 0, sizeof(double) * nres, c->stream) != cudaSuccess) return done(fail(QB_ERR_CUDA, "memset"));
+  if ((rc = run_pauli_sum(psi, lam, hlx, hlz, hc, dres + idx.size(), &nl)) != QB_OK) return done(rc);
+  if ((rc = run_pauli_adjoint(psi, lam, lx, lz, cs, dres)) != QB_OK) return done(rc);
+  std::vector<double> v(idx.size() + 1);
+  std::vector<double> host(nres);
+  if (cudaMemcpyAsync(host.data(), dres, sizeof(double) * nres, cudaMemcpyDeviceToHost, c->stream) != cudaSuccess ||
+      cudaStreamSynchronize(c->stream) != cudaSuccess)
+    return done(fail(QB_ERR_CUDA, "gradient read-back"));
+  for (size_t i = 0; i < idx.size(); ++i) v[i] = host[i];
+  double e = 0.0;
+  for (int l = 0; l < nl; ++l) e += host[idx.size() + l];  // (launch order: fixed)
+  v[idx.size()] = e;
+  if (c->nranks > 1) {
+    rc = dist_allreduce_sum(c->dist, v.data(), (int)v.size(), c->stream);
+    if (rc != QB_OK) return done(fail(rc, "allreduce failed: %s", dist_last_error()));
+  }
+  // the pending scalar z of psi, arithmetically: psi = z psi_dev, so both scale by |z|^2
+  const double g2 = psi->pscale[0] * psi->pscale[0] + psi->pscale[1] * psi->pscale[1];
+  for (size_t i = 0; i < idx.size(); ++i) grad[idx[i]] = v[i] * g2;
+  *energy = v[idx.size()] * g2;
+  return done(QB_OK);
 }
 
 int qb_normalize(qb_state *s) {

@@ -1315,6 +1315,241 @@ cudaError_t launch_pauli_rot(double2 *amps, int local_bits, const PauliRotArgs &
   return cudaGetLastError();
 }
 
+// ---------------------------------------------------------------- Pauli sums and the adjoint gradient
+// Both kernels use the tiles of k_pauli_rot_tile (the run's X bits topped up with the lowest local bits, loaded
+// with cp.async into swizzled shared memory, thread t owning tile-local indices t + k * threads), but a fixed
+// grid walks the tiles in a fixed order (tile blockIdx.x, + gridDim.x, ...): per-block partials then stay few
+// and the sums they feed are deterministic.
+template <class A>
+__device__ __forceinline__ uint64_t pauli_tile_base(const A &a, uint64_t t) {  // tile number -> its non-tile bits
+  uint64_t base = 0;
+  for (uint32_t i = 0; i < a.nruns; ++i) {
+    base |= (t & ((1ull << a.run_len[i]) - 1ull)) << a.run_shift[i];
+    t >>= a.run_len[i];
+  }
+  return base;
+}
+
+// offset inside the tile of the thread's k-th tile-local index tid + (k << THR)
+template <int TB, int THR>
+struct PauliTileMap {
+  uint64_t lo, hi[TB - THR];
+  template <class A>
+  __device__ __forceinline__ PauliTileMap(const A &a, uint32_t tid) {
+    lo = 0;
+#pragma unroll
+    for (int b = 0; b < THR; ++b)
+      if (b < (int)a.tile_bits && ((tid >> b) & 1u)) lo |= 1ull << a.tile_pos[b];
+#pragma unroll
+    for (int b = 0; b < TB - THR; ++b) hi[b] = b + THR < (int)a.tile_bits ? 1ull << a.tile_pos[b + THR] : 0ull;
+  }
+  __device__ __forceinline__ uint64_t at(int k) const {
+    uint64_t o = lo;
+#pragma unroll
+    for (int b = 0; b < TB - THR; ++b)
+      if ((k >> b) & 1) o |= hi[b];
+    return o;
+  }
+};
+
+__device__ __forceinline__ void cp_async16(void *smem, const void *gmem) {
+  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(uint32_t(__cvta_generic_to_shared(smem))), "l"(gmem)
+               : "memory");
+}
+
+// out (+)= H_run src over one tile per step.  The tile of src is read by every thread after one barrier; each
+// thread then sums the run's terms for its own indices without further barriers.
+template <int TB>
+__global__ void __launch_bounds__(kPauliThreads, 3) k_pauli_sum_tile(const double2 *__restrict__ src, double2 *__restrict__ out,
+                                                                    const __grid_constant__ PauliSumArgs a, uint64_t ntiles,
+                                                                    double *__restrict__ partials) {
+  constexpr int kThrBits = 8;
+  static_assert(kPauliThreads == 1 << kThrBits && TB > kThrBits, "tile-local index = thread + k * kPauliThreads");
+  constexpr int EPT = 1 << (TB - kThrBits);
+  extern __shared__ double2 tile[];
+  const uint32_t tid = threadIdx.x, nel = 1u << a.tile_bits, nterms = a.nterms;
+  const PauliTileMap<TB, kThrBits> map(a, tid);
+  double acc[1] = {0.0};
+  for (uint64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
+    const uint64_t base = pauli_tile_base(a, t);
+#pragma unroll
+    for (int k = 0; k < EPT; ++k)
+      if (tid + k * kPauliThreads < nel) cp_async16(tile + swz(tid + k * kPauliThreads), src + (base | map.at(k)));
+    asm volatile("cp.async.wait_all;" ::: "memory");
+    __syncthreads();
+#pragma unroll 2
+    for (int k = 0; k < EPT; ++k) {
+      const uint32_t u = tid + k * kPauliThreads;
+      if (u >= nel) continue;
+      double hr = 0.0, hi = 0.0;
+      for (uint32_t i = 0; i < nterms; ++i) {
+        const PauliSumParam &p = a.term[i];
+        const uint32_t v = u ^ p.xt;
+        const double2 w = tile[swz(v)];
+        const bool neg = (uint32_t(__popc(v & p.zt)) ^ uint32_t(__popcll(base & p.zout))) & 1u;
+        const double cr = neg ? -p.cr : p.cr, ci = neg ? -p.ci : p.ci;
+        hr = fma(cr, w.x, fma(-ci, w.y, hr));
+        hi = fma(cr, w.y, fma(ci, w.x, hi));
+      }
+      if (partials) {
+        const double2 s = tile[swz(u)];
+        acc[0] = fma(s.x, hr, fma(s.y, hi, acc[0]));
+      }
+      const uint64_t g = base | map.at(k);
+      if (!a.first) {
+        const double2 o = __ldcs(out + g);
+        hr += o.x;
+        hi += o.y;
+      }
+      __stcs(out + g, make_double2(hr, hi));
+    }
+    __syncthreads();  // the next tile's load overwrites what other threads read
+  }
+  if (partials) block_reduce_store<1>(acc, partials + blockIdx.x);
+}
+
+// Rotations nrot-1 .. 0 undone on tiles of psi and lam, each rotation's part of Im <lam|P|psi> taken first.
+// A rotation with X is one pair per thread and iteration after a barrier; a Z-only rotation is per amplitude
+// over the thread's own indices and needs none after a Z-only step.  The per-rotation sums go through warp
+// shuffles into this warp's row of wpart (each row written by one lane only, tiles in a fixed order), and the
+// rows are added in a fixed order at the end.
+template <int TB>
+__global__ void __launch_bounds__(kPauliAdjThreads, 1)
+    k_pauli_rot_adjoint_tile(double2 *__restrict__ psi, double2 *__restrict__ lam, const __grid_constant__ PauliAdjArgs a,
+                             uint64_t ntiles, double *__restrict__ partials) {
+  constexpr int kThrBits = 9, kWarps = kPauliAdjThreads / 32;
+  static_assert(kPauliAdjThreads == 1 << kThrBits && TB > kThrBits, "tile-local index = thread + k * kPauliAdjThreads");
+  constexpr int EPT = 1 << (TB - kThrBits);
+  extern __shared__ double2 smem[];
+  __shared__ double wpart[kWarps][kPauliMaxRot];
+  double2 *const tp = smem, *const tl = smem + (1 << TB);
+  const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5, nel = 1u << a.tile_bits, nrot = a.nrot;
+  for (uint32_t r = lane; r < (uint32_t)kPauliMaxRot; r += 32) wpart[warp][r] = 0.0;
+  __syncwarp();
+  const PauliTileMap<TB, kThrBits> map(a, tid);
+  for (uint64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
+    const uint64_t base = pauli_tile_base(a, t);
+#pragma unroll
+    for (int k = 0; k < EPT; ++k)
+      if (tid + k * kPauliAdjThreads < nel) {
+        const uint32_t su = swz(tid + k * kPauliAdjThreads);
+        const uint64_t g = base | map.at(k);
+        cp_async16(tp + su, psi + g);
+        cp_async16(tl + su, lam + g);
+      }
+    asm volatile("cp.async.wait_all;" ::: "memory");  // (own indices: visible to this thread, no barrier)
+    bool own = true;
+    for (int r = int(nrot) - 1; r >= 0; --r) {
+      const PauliAdjParam &p = a.rot[r];
+      const uint32_t s0 = uint32_t(__popcll(base & p.zout)) & 1u;
+      double part = 0.0;
+      if (p.xt == 0) {
+        if (!own) __syncthreads();
+#pragma unroll 2
+        for (int k = 0; k < EPT; ++k) {
+          const uint32_t u = tid + k * kPauliAdjThreads;
+          if (u >= nel) continue;
+          const bool neg = (uint32_t(__popc(u & p.zt)) ^ s0) & 1u;
+          const double fr = neg ? -p.fr : p.fr, fi = neg ? -p.fi : p.fi;
+          const double2 A = tp[swz(u)], LA = tl[swz(u)];
+          const double pr = fr * A.x - fi * A.y, pi = fr * A.y + fi * A.x;      // (P psi)_u
+          const double lr = fr * LA.x - fi * LA.y, li = fr * LA.y + fi * LA.x;  // (P lam)_u
+          part = fma(LA.x, pi, fma(-LA.y, pr, part));
+          tp[swz(u)] = make_double2(p.c * A.x - p.s * pi, p.c * A.y + p.s * pr);
+          tl[swz(u)] = make_double2(p.c * LA.x - p.s * li, p.c * LA.y + p.s * lr);
+        }
+        own = true;
+      } else {
+        __syncthreads();
+        const uint32_t h = 31 - __clz(p.xt), lo = (1u << h) - 1u;  // pairs (j, j ^ xt), bit h of j clear
+#pragma unroll 2
+        for (int k = 0; k < EPT / 2; ++k) {
+          const uint32_t q = tid + k * kPauliAdjThreads;
+          if (q >= nel / 2) continue;
+          const uint32_t j = ((q & ~lo) << 1) | (q & lo), jx = j ^ p.xt;
+          const bool nj = (uint32_t(__popc(j & p.zt)) ^ s0) & 1u, nk = (uint32_t(__popc(jx & p.zt)) ^ s0) & 1u;
+          // (P v)_j = f (-1)^[jx] v_jx and (P v)_jx = f (-1)^[j] v_j
+          const double ajr = nk ? -p.fr : p.fr, aji = nk ? -p.fi : p.fi, akr = nj ? -p.fr : p.fr, aki = nj ? -p.fi : p.fi;
+          const double2 A = tp[swz(j)], B = tp[swz(jx)], LA = tl[swz(j)], LB = tl[swz(jx)];
+          const double par = ajr * B.x - aji * B.y, pai = ajr * B.y + aji * B.x;
+          const double pbr = akr * A.x - aki * A.y, pbi = akr * A.y + aki * A.x;
+          const double lar = ajr * LB.x - aji * LB.y, lai = ajr * LB.y + aji * LB.x;
+          const double lbr = akr * LA.x - aki * LA.y, lbi = akr * LA.y + aki * LA.x;
+          part = fma(LA.x, pai, fma(-LA.y, par, part));
+          part = fma(LB.x, pbi, fma(-LB.y, pbr, part));
+          tp[swz(j)] = make_double2(p.c * A.x - p.s * pai, p.c * A.y + p.s * par);
+          tp[swz(jx)] = make_double2(p.c * B.x - p.s * pbi, p.c * B.y + p.s * pbr);
+          tl[swz(j)] = make_double2(p.c * LA.x - p.s * lai, p.c * LA.y + p.s * lar);
+          tl[swz(jx)] = make_double2(p.c * LB.x - p.s * lbi, p.c * LB.y + p.s * lbr);
+        }
+        own = false;
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) part += __shfl_down_sync(0xffffffffu, part, o);
+      if (lane == 0) wpart[warp][r] += part;
+    }
+    if (!own) __syncthreads();
+#pragma unroll
+    for (int k = 0; k < EPT; ++k)
+      if (tid + k * kPauliAdjThreads < nel) {
+        const uint32_t su = swz(tid + k * kPauliAdjThreads);
+        const uint64_t g = base | map.at(k);
+        __stcs(psi + g, tp[su]);
+        __stcs(lam + g, tl[su]);
+      }
+  }
+  __syncthreads();
+  if (tid < nrot) {
+    double s = 0.0;
+    for (int w = 0; w < kWarps; ++w) s += wpart[w][tid];
+    partials[size_t(blockIdx.x) * kPauliMaxRot + tid] = s;
+  }
+}
+
+// the fixed grid of a tile-walking kernel: every CTA an SM holds, capped at the number of tiles
+template <class F>
+static cudaError_t pauli_walk_grid(F fn, int threads, size_t smem, uint64_t ntiles, int sm_count, int *grid) {
+  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
+  if (e != cudaSuccess) return e;
+  int per_sm = 0;
+  e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, fn, threads, smem);
+  if (e != cudaSuccess) return e;
+  if (per_sm < 1) return cudaErrorInvalidConfiguration;
+  *grid = (int)std::min<uint64_t>(ntiles, uint64_t(sm_count) * per_sm);
+  return cudaSuccess;
+}
+
+cudaError_t launch_pauli_sum(const double2 *src, double2 *out, int local_bits, const PauliSumArgs &args,
+                             double *partials_dev, double *energy_dev, int sm_count, cudaStream_t stream) {
+  if (args.nterms < 1 || args.nterms > (uint32_t)kPauliMaxRot || args.tile_bits > (uint32_t)kPauliTileBits ||
+      (int)args.tile_bits > local_bits || (partials_dev && !energy_dev))
+    return cudaErrorInvalidValue;
+  const auto fn = k_pauli_sum_tile<kPauliTileBits>;
+  const uint64_t ntiles = 1ull << (local_bits - args.tile_bits);
+  int g = 0;
+  cudaError_t e = pauli_walk_grid(fn, kPauliThreads, sizeof(double2) << kPauliTileBits, ntiles, sm_count, &g);
+  if (e != cudaSuccess) return e;
+  fn<<<g, kPauliThreads, sizeof(double2) << args.tile_bits, stream>>>(src, out, args, ntiles, partials_dev);
+  if (partials_dev) k_expect_final<<<1, kRedThreads, 0, stream>>>(partials_dev, g, 1, energy_dev);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_pauli_rot_adjoint(double2 *psi, double2 *lam, int local_bits, const PauliAdjArgs &args,
+                                     double *partials_dev, double *grad_dev, int sm_count, cudaStream_t stream) {
+  if (args.nrot < 1 || args.nrot > (uint32_t)kPauliMaxRot || args.tile_bits > (uint32_t)kPauliTileBits ||
+      (int)args.tile_bits > local_bits)
+    return cudaErrorInvalidValue;
+  const auto fn = k_pauli_rot_adjoint_tile<kPauliTileBits>;
+  const uint64_t ntiles = 1ull << (local_bits - args.tile_bits);
+  int g = 0;
+  cudaError_t e = pauli_walk_grid(fn, kPauliAdjThreads, 2 * (sizeof(double2) << kPauliTileBits), ntiles, sm_count, &g);
+  if (e != cudaSuccess) return e;
+  fn<<<g, kPauliAdjThreads, 2 * (sizeof(double2) << kPauliTileBits), stream>>>(psi, lam, args, ntiles, partials_dev);
+  // partials[block][kPauliMaxRot]: one block of the final stage per rotation
+  k_expect_final<<<args.nrot, kRedThreads, 0, stream>>>(partials_dev, g, kPauliMaxRot, grad_dev);
+  return cudaGetLastError();
+}
+
 // ---------------------------------------------------------------- live sub-cube kernels
 // After a collapse (StateVec.hs:104-114) half of the state is exactly zero, and a fresh
 // |0...0> is zero outside one amplitude.  The host tracks the index bits whose value is KNOWN

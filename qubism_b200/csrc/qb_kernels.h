@@ -77,6 +77,45 @@ struct PauliRotArgs {
 };
 cudaError_t launch_pauli_rot(double2 *amps, int local_bits, const PauliRotArgs &args, cudaStream_t stream);
 
+// A Pauli sum applied to a state (qb_pauli_sum): out (+)= sum_t (cr + i ci)_t (-1)^popc((j ^ xt) & zt)
+// (-1)^popc(base & zout) src_(j ^ xt) for up to kPauliMaxRot terms whose X bits fit one tile (the tile geometry
+// of PauliRotArgs).  first != 0: out is stored, else added to.  partials != null: each block also leaves
+// Re sum_j conj(src_j) (this launch's part of out)_j in partials[block], reduced into *energy_dev in a fixed
+// order.  A fixed grid walks the tiles in a fixed order: deterministic.
+struct PauliSumParam {
+  uint64_t zout;
+  double cr, ci;      // the term's coefficient times i^popc(x & z) and the sign of Z on global qubits
+  uint32_t xt, zt;
+};
+struct PauliSumArgs {
+  uint32_t nterms, tile_bits, nruns, first;
+  uint8_t tile_pos[16];
+  uint8_t run_shift[16], run_len[16];
+  PauliSumParam term[kPauliMaxRot];
+};
+cudaError_t launch_pauli_sum(const double2 *src, double2 *out, int local_bits, const PauliSumArgs &args,
+                             double *partials_dev, double *energy_dev, int sm_count, cudaStream_t stream);
+
+// The backward pass of the adjoint gradient (qb_pauli_rot_grad) over one launch of rotations: psi and lam
+// (same layout) are walked through rotations nrot-1 .. 0; for each, grad_dev[r] = Im sum_j conj(lam_j) (P_r psi)_j,
+// then psi <- R_r^dagger psi and lam <- R_r^dagger lam with R_r^dagger = c I + i s P_r.  (P psi)_j =
+// (fr + i fi) (-1)^popc((j ^ xt) & zt) (-1)^popc(base & zout) psi_(j ^ xt).  Per-block partials of each rotation
+// are reduced in a fixed order (partials[block * kPauliMaxRot + r]), then into grad_dev by k_expect_final.
+constexpr int kPauliAdjThreads = 512;
+struct PauliAdjParam {
+  uint64_t zout;
+  double c, s, fr, fi;
+  uint32_t xt, zt;
+};
+struct PauliAdjArgs {
+  uint32_t nrot, tile_bits, nruns, _pad;
+  uint8_t tile_pos[16];
+  uint8_t run_shift[16], run_len[16];
+  PauliAdjParam rot[kPauliMaxRot];
+};
+cudaError_t launch_pauli_rot_adjoint(double2 *psi, double2 *lam, int local_bits, const PauliAdjArgs &args,
+                                     double *partials_dev, double *grad_dev, int sm_count, cudaStream_t stream);
+
 // Live sub-cube {i : i & fixed_mask == fixed_val} of the shard (see "support" in qb_api.cpp): the
 // reduction of launch_sumsq restricted to it, and zero-fill (mode 0) / scaling (mode 1) of it.
 int cube_runs(int local_bits, uint64_t fixed_mask);  // must be <= kMaxRuns for the launchers below

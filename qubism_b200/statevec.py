@@ -326,6 +326,42 @@ class StateVec:
                                                  th.ctypes.data_as(C.POINTER(C.c_double)), len(xs)))
         return self
 
+    def pauli_sum(self, terms, coefs) -> "StateVec":
+        """``(sum_t coefs[t] P_t) #> self`` as a NEW state (qb_pauli_sum); ``self`` keeps its value.  Terms are
+        spelled as for ``expect_pauli``; coefficients may be complex.  Duplicate strings add; no terms: zero."""
+        xs, zs = pauli_masks(terms, self.n)
+        cf = np.ascontiguousarray(coefs, dtype=np.complex128).reshape(-1)
+        if cf.size != xs.size:
+            raise ValueError(f"{xs.size} Pauli strings but {cf.size} coefficients")
+        P64 = C.POINTER(C.c_uint64)
+        h = C.c_void_p()
+        capi.check(self.ctx.L.qb_pauli_sum(self._h, xs.ctypes.data_as(P64), zs.ctypes.data_as(P64),
+                                           cf.ctypes.data_as(C.c_void_p), len(xs), C.byref(h)))
+        return StateVec(h, self.ctx)
+
+    def pauli_rot_grad(self, rot_terms, thetas, h_terms, h_coefs):
+        """Energy and gradient of ``E(theta) = sum_t h_coefs[t] realPart (psi <.> (H_t #> psi))`` with
+        ``psi = exp(-i theta_{K-1}/2 P_{K-1}) ... exp(-i theta_0/2 P_0) #> self`` (qb_pauli_rot_grad, the adjoint
+        method).  Terms are spelled as for ``expect_pauli``; ``h_coefs`` are real.  ``self`` keeps its value.
+        Returns ``(energy, grad)`` with ``grad[k] = dE / dtheta_k`` as float64[K]."""
+        n = self.n
+        rx, rz = pauli_masks(rot_terms, n)
+        hx, hz = pauli_masks(h_terms, n)
+        th = np.ascontiguousarray(thetas, dtype=np.float64).reshape(-1)
+        hc = np.ascontiguousarray(h_coefs, dtype=np.float64).reshape(-1)
+        if th.size != rx.size:
+            raise ValueError(f"{rx.size} rotation strings but {th.size} angles")
+        if hc.size != hx.size:
+            raise ValueError(f"{hx.size} Pauli strings but {hc.size} coefficients")
+        grad = np.zeros(rx.size, dtype=np.float64)
+        energy = C.c_double()
+        P64, PD = C.POINTER(C.c_uint64), C.POINTER(C.c_double)
+        capi.check(self.ctx.L.qb_pauli_rot_grad(self._h, rx.ctypes.data_as(P64), rz.ctypes.data_as(P64),
+                                                th.ctypes.data_as(PD), len(rx), hx.ctypes.data_as(P64),
+                                                hz.ctypes.data_as(P64), hc.ctypes.data_as(PD), len(hx),
+                                                C.byref(energy), grad.ctypes.data_as(PD)))
+        return energy.value, grad
+
     def norm(self) -> float:  # Algebra.hs:35-36: realPart (a <.> a), the SQUARED norm
         return self.inner(self).real
 
@@ -413,3 +449,13 @@ def pauliRotate(terms, thetas, sv: StateVec) -> StateVec:
     """``exp(-i theta_k/2 P_k) ... exp(-i theta_0/2 P_0) #> sv`` as a new value; ``sv`` keeps its own
     (a lazy clone rotated in place, see StateVec.pauli_rot_)."""
     return sv.clone().pauli_rot_(terms, thetas)
+
+
+def pauliSum(terms, coefs, sv: StateVec) -> StateVec:
+    """``(sum_t coefs[t] P_t) #> sv`` as a new value (see StateVec.pauli_sum)."""
+    return sv.pauli_sum(terms, coefs)
+
+
+def pauliRotGrad(rot_terms, thetas, h_terms, h_coefs, sv: StateVec):
+    """``(energy, grad)`` of a Pauli-sum energy over Pauli rotations of ``sv`` (see StateVec.pauli_rot_grad)."""
+    return sv.pauli_rot_grad(rot_terms, thetas, h_terms, h_coefs)
