@@ -59,3 +59,5 @@ foreign import ccall safe   "qb_apply_pauli_rot" c_qb_apply_pauli_rot :: Ptr QbS
 -- Pauli sums and adjoint gradients ------------------------------------------------------------
 foreign import ccall safe   "qb_pauli_sum"       c_qb_pauli_sum       :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Ptr C -> Int64 -> Ptr (Ptr QbState) -> IO CInt
 foreign import ccall safe   "qb_pauli_rot_grad"  c_qb_pauli_rot_grad  :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Ptr CDouble -> Int64 -> Ptr Word64 -> Ptr Word64 -> Ptr CDouble -> Int64 -> Ptr CDouble -> Ptr CDouble -> IO CInt
+-- exact time evolution under Pauli sums ------------------------------------------------------
+foreign import ccall safe   "qb_pauli_evolve"    c_qb_pauli_evolve    :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Ptr CDouble -> Int64 -> CDouble -> Ptr Int64 -> IO CInt

@@ -1,7 +1,8 @@
 {-|
 Module      : Qubism.Expect
-Description : expectation values of Pauli strings, Pauli rotations, Pauli sums and adjoint gradients,
-              computed on the device (qb_expect_pauli, qb_apply_pauli_rot, qb_pauli_sum, qb_pauli_rot_grad)
+Description : expectation values of Pauli strings, Pauli rotations, Pauli sums, adjoint gradients and exact
+              time evolution, computed on the device (qb_expect_pauli, qb_apply_pauli_rot, qb_pauli_sum,
+              qb_pauli_rot_grad, qb_pauli_evolve)
 
 @expectPauli terms sv@ is @[realPart (sv <.> (p #> sv)) | p <- terms]@ for the Pauli strings @p@ that
 @terms@ name (QGate.hs:90-108 for pauliX / pauliY / pauliZ), without building any @p #> sv@: one
@@ -16,8 +17,11 @@ run of rotations whose X qubits fit one tile together.
 
 @pauliRotGrad rots h sv@ is @(e, grad)@ with @e = sum_t h_t realPart (psi <.> (p_t #> psi))@ for
 @psi = pauliRotate rots sv@ and @grad !! k = d e / d theta_k@ (the adjoint method: about one forward pass,
-one @pauliSum@ and one backward pass, whatever the number of angles).  UNVERIFIED BY COMPILATION (no GHC in
-the build image).
+one @pauliSum@ and one backward pass, whatever the number of angles).
+
+@pauliEvolve h t sv@ is @exp (-i t H) #> sv@ for @H = sum_t h_t p_t@ (real coefficients), as a new value: a
+Chebyshev expansion exact to double precision (clone + in-place evolution).  UNVERIFIED BY COMPILATION (no
+GHC in the build image).
 -}
 {-# LANGUAGE DataKinds, KindSignatures, ScopedTypeVariables #-}
 module Qubism.Expect
@@ -26,6 +30,7 @@ module Qubism.Expect
   , pauliRotate
   , pauliSum
   , pauliRotGrad
+  , pauliEvolve
   ) where
 
 import GHC.TypeLits
@@ -86,6 +91,17 @@ pauliRotGrad rots h sv = unsafePerformIO $
     (rxs, rzs) = unzip (map masks rterms)
     (hterms, hcs) = unzip h
     (hxs, hzs) = unzip (map masks hterms)
+
+-- | Real coefficients: H is Hermitian.  The same strings are errors as for pauliRotate.
+pauliEvolve :: KnownNat n => [([(Finite n, Pauli)], Double)] -> Double -> StateVec n -> StateVec n
+pauliEvolve h t sv = unsafePerformIO $ do
+  r <- cloneSV sv
+  withArrayLen xs $ \k px -> withArray zs $ \pz -> withArray (map realToFrac hcs) $ \pc -> withSV r $ \p -> do
+    rc <- c_qb_pauli_evolve p px pz pc (fromIntegral k) (realToFrac t) nullPtr
+    if rc /= 0 then error ("qubism_sv: status " ++ show rc) else pure r
+  where
+    (terms, hcs) = unzip h
+    (xs, zs) = unzip (map masks terms)
 
 -- bit q of the X / Z mask = qubit q: X = x only, Z = z only, Y = both
 masks :: [(Finite n, Pauli)] -> (Word64, Word64)

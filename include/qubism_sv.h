@@ -247,6 +247,32 @@ int qb_pauli_rot_grad(qb_state *s, const uint64_t *rx, const uint64_t *rz, const
                       const uint64_t *hx, const uint64_t *hz, const double *hcoef, int64_t nterms, double *energy,
                       double *grad);
 
+/* ---- exact time evolution under Pauli sums ---------------------------------------------- */
+/* s <- exp(-i t H) s, H = sum_t hcoef[t] P_t (strings as qb_expect_pauli, real coefficients: H is Hermitian).
+ * Equal strings add, zero coefficients drop out, and the identity strings are the global phase e^{-itc}
+ * (c = their coefficients' sum).  The rest is a Chebyshev expansion in H' = (H - c) / r, r = sum |h| over the
+ * merged non-identity strings, tau = t r:
+ *   exp(-itH) s = e^{-itc} sum_{k=0..K} a_k T_k(H') s,  a_0 = J_0(tau), a_k = 2 (-i)^k J_k(tau),
+ * K the smallest k >= 1 with 2 sum_{j>k} |J_j(tau)| <= 2^-53 (the a-priori truncation bound, ||T_k(H')|| <= 1):
+ * 14 steps at tau = 1, 136 at tau = 87, 975 at tau = 870.  *nsteps (may be null) = K; 0 when nothing runs.
+ * Observes s (flushes its queued gates) and runs at once; s changes value in place: lazy clones of the older
+ * value keep it (copy-on-write), and with option "linear" = 1 they are consumed as by any in-place change.
+ * t = 0 or nterms = 0: nothing happens.  An H without non-identity strings only multiplies the deferred
+ * scalar, like qb_scale (nothing is launched).  The pending scalar of s carries through (the map is linear;
+ * a non-finite one is forced into the data first).  The result knows the qubits of known value that s knew
+ * outside every non-identity X mask.  Deterministic (no reductions).  Distributed: a collective.
+ * Cost: K steps, each one launch per run of the cut qb_pauli_sum makes for the merged non-identity strings
+ * (simple_launches grows by K times those launches); each launch reads T_k and T_{k-1} and writes T_{k+1},
+ * the step's last also updates the sum.  Memory: two temporary states besides s.
+ * Everything is checked before anything is queued, allocated or written (a rejected call leaves s and its
+ * queue untouched):
+ * QB_ERR_ARG: a null pointer with nterms > 0, nterms < 0, a mask bit at or above n, a non-finite coefficient
+ * or t, or K over 2^20 (|t| r up to about 10^6).  QB_ERR_UNSUPPORTED: X / Y on more than QB_PAULI_ROT_MAX_X
+ * qubits, or on more qubits than a shard holds.  QB_ERR_OOM: no room for the temporaries (s stays valid and
+ * unchanged). */
+int qb_pauli_evolve(qb_state *s, const uint64_t *hx, const uint64_t *hz, const double *hcoef, int64_t nterms,
+                    double t, int64_t *nsteps);
+
 /* ---- introspection (tests, bench, profiling) ------------------------------------------- */
 typedef struct {
   uint64_t ops_submitted;   /* primitive ops received through the ABI                     */

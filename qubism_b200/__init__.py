@@ -8,6 +8,6 @@ from . import capi  # noqa: F401
 from .qgate import (QGate, apply, cnot, controlled, gate, hadamard, ident, ifBit, kronecker, onEvery, onJust,  # noqa: F401
                     onRange, pauliX, pauliY, pauliZ, unitary, unitary_matrix)
 from .statevec import (Context, StateVec, collapse, dimension, expectPauli, measure, measureQubit, mkQubit,  # noqa: F401
-                       mkStateVec, normalize, pauliRotate, pauliRotGrad, pauliSum, tensor, zero)
+                       mkStateVec, normalize, pauliEvolve, pauliRotate, pauliRotGrad, pauliSum, tensor, zero)
 
 __version__ = "0.1.0"

@@ -1443,52 +1443,146 @@ void pauli_phase(const Buffer *s, uint64_t lx, uint64_t lz, double re, double im
   }
 }
 
-// out <- (sum_t coef[t] P_t) src, P_t named by logical masks; out is a fresh shard of src's size whose old
-// contents do not matter.  Terms are taken in the order of their X masks (a sum commutes; a stable sort, so
-// the order is a fixed function of the input) and cut by pauli_cut.  The first launch writes every amplitude
-// of out in src's layout; later launches add, out following src's layout (localise_x) by relayout.
-// energy_dev: Re <src| H_launch src> of launch l into energy_dev[l], *nlaunch = the number of launches.
+// Pauli-sum terms named by logical masks (coef: (re, im) per term), taken in the order of their X masks (a sum
+// commutes; a stable sort, so the order is a fixed function of the input): the i-th is term ord[i], its X mask
+// sx[i].  run_pauli_sum and the Chebyshev steps of qb_pauli_evolve cut them alike.
+struct PauliTerms {
+  std::vector<uint64_t> lx, lz;
+  std::vector<double> coef;
+  std::vector<size_t> ord;
+  std::vector<uint64_t> sx;
+  PauliTerms(std::vector<uint64_t> x, std::vector<uint64_t> z, std::vector<double> cf)
+      : lx(std::move(x)), lz(std::move(z)), coef(std::move(cf)), ord(lx.size()), sx(lx.size()) {
+    for (size_t t = 0; t < ord.size(); ++t) ord[t] = t;
+    std::stable_sort(ord.begin(), ord.end(), [&](size_t a, size_t b) { return lx[a] < lx[b]; });
+    for (size_t t = 0; t < ord.size(); ++t) sx[t] = lx[ord[t]];
+  }
+};
+
+// The launch of a Pauli sum that starts at sorted term i0: cut by pauli_cut on src's layout, its X qubits brought
+// into src's shard (sharded), and its tile and terms filled in for src's layout with the coefficients scaled by
+// f.  *i1 = the end of the launch.
+int pauli_sum_launch(Buffer *src, const PauliTerms &h, double f, size_t i0, size_t *i1, PauliSumArgs &args) {
+  qb_ctx *c = src->ctx;
+  uint64_t ux = 0;
+  *i1 = pauli_cut(src, h.sx, i0, &ux);
+  if (c->nranks > 1) QB_TRY(localise_x(src, ux));
+  const uint64_t local = (1ull << src->L) - 1ull;
+  memset(&args, 0, sizeof args);
+  args.nterms = uint32_t(*i1 - i0);
+  QB_TRY(pauli_tile(src, ux, args));
+  uint64_t tile = 0;
+  for (uint32_t i = 0; i < args.tile_bits; ++i) tile |= 1ull << args.tile_pos[i];
+  for (size_t i = i0; i < *i1; ++i) {
+    const size_t t = h.ord[i];
+    const uint64_t zp = phys_mask(src, h.lz[t]);
+    PauliSumParam &p = args.term[i - i0];
+    p.xt = pauli_tile_local(args, phys_mask(src, h.lx[t]));
+    p.zt = pauli_tile_local(args, zp);
+    p.zout = zp & local & ~tile;
+    pauli_phase(src, h.lx[t], h.lz[t], f * h.coef[2 * t], f * h.coef[2 * t + 1], &p.cr, &p.ci);
+  }
+  return QB_OK;
+}
+
+// out <- (sum_t coef[t] P_t) src; out is a fresh shard of src's size whose old contents do not matter.  The first
+// launch writes every amplitude of out in src's layout; later launches add, out following src's layout
+// (localise_x) by relayout.  energy_dev: Re <src| H_launch src> of launch l into energy_dev[l], *nlaunch = the
+// number of launches.
 int run_pauli_sum(Buffer *src, Buffer *out, const std::vector<uint64_t> &lx, const std::vector<uint64_t> &lz,
                   const std::vector<double> &coef, double *energy_dev, int *nlaunch) {
   qb_ctx *c = src->ctx;
   QB_TRY(ensure_inplace(src));
-  const uint64_t local = (1ull << src->L) - 1ull;
-  std::vector<size_t> ord(lx.size());
-  for (size_t t = 0; t < ord.size(); ++t) ord[t] = t;
-  std::stable_sort(ord.begin(), ord.end(), [&](size_t a, size_t b) { return lx[a] < lx[b]; });
-  std::vector<uint64_t> sx(ord.size());
-  for (size_t t = 0; t < ord.size(); ++t) sx[t] = lx[ord[t]];
+  const PauliTerms h(lx, lz, coef);
   int nl = 0;
-  for (size_t i0 = 0; i0 < sx.size(); ++nl) {
-    uint64_t ux = 0;
-    const size_t i1 = pauli_cut(src, sx, i0, &ux);
-    if (c->nranks > 1) QB_TRY(localise_x(src, ux));
+  for (size_t i0 = 0, i1 = 0; i0 < h.sx.size(); ++nl, i0 = i1) {
+    PauliSumArgs args;
+    QB_TRY(pauli_sum_launch(src, h, 1.0, i0, &i1, args));
     if (nl == 0) out->perm = src->perm;  // (the first launch writes every amplitude: born in src's layout)
     else if (out->perm != src->perm) QB_TRY(relayout(out, src->perm));
-    PauliSumArgs args;
-    memset(&args, 0, sizeof args);
-    args.nterms = uint32_t(i1 - i0);
     args.first = nl == 0;
-    QB_TRY(pauli_tile(src, ux, args));
-    uint64_t tile = 0;
-    for (uint32_t i = 0; i < args.tile_bits; ++i) tile |= 1ull << args.tile_pos[i];
-    for (size_t i = i0; i < i1; ++i) {
-      const size_t t = ord[i];
-      const uint64_t zp = phys_mask(src, lz[t]);
-      PauliSumParam &p = args.term[i - i0];
-      p.xt = pauli_tile_local(args, phys_mask(src, lx[t]));
-      p.zt = pauli_tile_local(args, zp);
-      p.zout = zp & local & ~tile;
-      pauli_phase(src, lx[t], lz[t], coef[2 * t], coef[2 * t + 1], &p.cr, &p.ci);
-    }
     QB_CUDA(launch_pauli_sum(src->amps, out->amps, src->L, args, energy_dev ? c->red_partials : nullptr,
                              energy_dev ? energy_dev + nl : nullptr, c->sm_count, c->stream));
     c->stats.simple_launches++;
     if (energy_dev) c->stats.reduce_launches++;
-    i0 = i1;
   }
   if (nlaunch) *nlaunch = nl;
   return QB_OK;
+}
+
+// Step k >= 1 of the Chebyshev recurrence of qb_pauli_evolve, one launch per run of the cut of h (H' = f h with
+// f = 1 / r; the terms are scaled by f at step 1 and by 2 f later): prev <- H' cur (step 1) or 2 H' cur - prev,
+// then acc <- a0 cur + ak prev (step 1) or acc + ak prev.  All three shards end in cur's layout; prev's and
+// acc's old contents do not matter at step 1 (their first write is a store).
+int run_pauli_cheb_step(Buffer *cur, Buffer *prev, Buffer *acc, const PauliTerms &h, double f, int64_t step,
+                        const double a0[2], const double ak[2]) {
+  qb_ctx *c = cur->ctx;
+  for (size_t i0 = 0, i1 = 0; i0 < h.sx.size(); i0 = i1) {
+    PauliChebArgs args;
+    QB_TRY(pauli_sum_launch(cur, h, step == 1 ? f : 2.0 * f, i0, &i1, args.sum));
+    const bool first = i0 == 0, last = i1 == h.sx.size();
+    if (step == 1 && first) prev->perm = cur->perm;
+    else if (prev->perm != cur->perm) QB_TRY(relayout(prev, cur->perm));
+    if (step == 1) {
+      if (last) acc->perm = cur->perm;  // (acc is first written, whole, by step 1's last launch)
+    } else if (acc->perm != cur->perm) {
+      QB_TRY(relayout(acc, cur->perm));
+    }
+    args.out_mode = !first ? kChebOutAdd : step == 1 ? kChebOutStore : kChebOutSub;
+    args.acc_mode = !last ? kChebAccNone : step == 1 ? kChebAccFirst : kChebAccAdd;
+    args.a0r = a0[0];
+    args.a0i = a0[1];
+    args.akr = ak[0];
+    args.aki = ak[1];
+    QB_CUDA(launch_pauli_cheb(cur->amps, prev->amps, acc->amps, cur->L, args, c->sm_count, c->stream));
+    c->stats.simple_launches++;
+  }
+  return QB_OK;
+}
+
+// The Chebyshev coefficients of exp(-i tau x) on [-1, 1]: a[k] = (re, im) of a_0 = J_0(tau), a_k = 2 (-i)^k J_k(tau)
+// for k = 0 .. K, K the smallest k >= 1 whose truncation bound 2 sum_{j > k} |J_j(tau)| is at most 2^-53.
+// J_k by Miller's backward recurrence from far above K (rescaled before it can overflow), normalised with
+// J_0 + 2 sum_m J_2m = 1; J_k(-tau) = (-1)^k J_k(tau).  false: K would exceed max_k.
+bool cheb_coefficients(double tau, int64_t max_k, std::vector<double> &a) {
+  const double at = std::fabs(tau);
+  if (!(at < double(max_k))) return false;  // (K > |tau| once |tau| is large: no need to look)
+  std::vector<double> J;
+  int64_t K = 1;
+  if (at < 0x1p-30) {  // J_0 = 1 - tau^2 / 4 and J_1 = tau / 2 to double precision; the tail ~ tau^2 / 4
+    J = {1.0, 0.5 * at};
+  } else {
+    const int64_t N = int64_t(std::ceil(at + 20.0 * std::cbrt(at))) + 40;
+    J.assign(size_t(N) + 2, 0.0);
+    J[N] = 1.0;
+    for (int64_t k = N; k >= 1; --k) {
+      J[k - 1] = (2.0 * double(k) / at) * J[k] - J[k + 1];
+      if (std::fabs(J[k - 1]) > 1e250)
+        for (int64_t j = k - 1; j <= N; ++j) J[j] *= 1e-250;
+    }
+    double norm = J[0];
+    for (int64_t k = 2; k <= N; k += 2) norm += 2.0 * J[k];
+    for (double &v : J) v /= norm;
+    double tail = 0.0;  // sum_{j > k} |J_j|, k falling
+    K = N;
+    for (int64_t k = N; k >= 1 && 2.0 * tail <= 0x1p-53; --k) {
+      K = k;
+      tail += std::fabs(J[k]);
+    }
+    if (K > N - 20) return false;  // (cannot happen: N lies far beyond the point where the tail is negligible)
+    if (K > max_k) return false;
+  }
+  a.assign(2 * size_t(K + 1), 0.0);
+  for (int64_t k = 0; k <= K; ++k) {
+    const double j = (tau < 0 && (k & 1)) ? -J[k] : J[k], m = k == 0 ? 1.0 : 2.0;
+    switch (k & 3) {  // (-i)^k
+      case 0: a[2 * k] = m * j; break;
+      case 1: a[2 * k + 1] = -m * j; break;
+      case 2: a[2 * k] = -m * j; break;
+      default: a[2 * k + 1] = m * j; break;
+    }
+  }
+  return true;
 }
 
 // The backward pass of the adjoint gradient: psi = the state after the rotations (lx, lz, cos / sin of
@@ -2363,6 +2457,116 @@ int qb_pauli_rot_grad(qb_state *s, const uint64_t *rx, const uint64_t *rz, const
   const double g2 = psi->pscale[0] * psi->pscale[0] + psi->pscale[1] * psi->pscale[1];
   for (size_t i = 0; i < idx.size(); ++i) grad[idx[i]] = v[i] * g2;
   *energy = v[idx.size()] * g2;
+  return done(QB_OK);
+}
+
+// ---- exact time evolution under Pauli sums
+constexpr int64_t kEvolveMaxSteps = int64_t(1) << 20;  // bounds the coefficient table and the time of one call
+
+int qb_pauli_evolve(qb_state *s, const uint64_t *hx, const uint64_t *hz, const double *hcoef, int64_t nterms, double t,
+                    int64_t *nsteps) {
+  if (nsteps) *nsteps = 0;
+  if (!s) return fail(QB_ERR_ARG, "null state");
+  if (nterms < 0) return fail(QB_ERR_ARG, "nterms %lld < 0", (long long)nterms);
+  if (nterms > 0 && (!hx || !hz || !hcoef)) return fail(QB_ERR_ARG, "null argument");
+  if (!std::isfinite(t)) return fail(QB_ERR_ARG, "t is not finite");
+  QB_TRY(check_pauli_strings(s, "term", "coefficient", hx, hz, hcoef, 1, nterms));
+  qb_ctx *c = s->ctx;
+  Guard g(c);
+  QB_TRY(check_state(s));
+  if (t == 0.0 || nterms == 0) return QB_OK;
+  // H = cid I + h: equal strings merged (caller order), zero coefficients dropped, the identity apart
+  double cid = 0.0, r = 0.0;
+  std::vector<uint64_t> lx, lz;
+  std::vector<double> cf;
+  std::map<std::pair<uint64_t, uint64_t>, size_t> seen;
+  for (int64_t k = 0; k < nterms; ++k) {
+    if (!(hx[k] | hz[k])) {
+      cid += hcoef[k];
+      continue;
+    }
+    const auto it = seen.emplace(std::make_pair(hx[k], hz[k]), lx.size());
+    if (it.second) {
+      lx.push_back(logical_mask(s->n, hx[k]));
+      lz.push_back(logical_mask(s->n, hz[k]));
+      cf.push_back(hcoef[k]);
+      cf.push_back(0.0);
+    } else {
+      cf[2 * it.first->second] += hcoef[k];
+    }
+  }
+  uint64_t xunion = 0;
+  size_t nh = 0;
+  for (size_t k = 0; k < lx.size(); ++k) {
+    if (cf[2 * k] == 0.0) continue;
+    r += std::fabs(cf[2 * k]);
+    xunion |= lx[k];
+    lx[nh] = lx[k];
+    lz[nh] = lz[k];
+    cf[2 * nh] = cf[2 * k];
+    ++nh;
+  }
+  lx.resize(nh);
+  lz.resize(nh);
+  cf.resize(2 * nh);
+  const double tc = t * cid;
+  if (!std::isfinite(tc)) return fail(QB_ERR_ARG, "t times the identity coefficient is not finite");
+  const double phase[2] = {std::cos(tc), -std::sin(tc)};  // e^{-itc}
+  if (r == 0.0) {  // H = cid I: a global phase, deferred like qb_scale
+    if (phase[0] == 1.0 && phase[1] == 0.0) return QB_OK;
+    LogOp o;
+    o.kind = LOG_SCALE;
+    o.m[0] = phase[0];
+    o.m[1] = phase[1];
+    return append(s, std::move(o));
+  }
+  const double tau = t * r;
+  std::vector<double> a;
+  if (!std::isfinite(tau) || !cheb_coefficients(tau, kEvolveMaxSteps, a))
+    return fail(QB_ERR_ARG, "|t| * sum |h| = %g needs more than %lld Chebyshev steps", std::fabs(tau),
+                (long long)kEvolveMaxSteps);
+  const int64_t K = int64_t(a.size() / 2) - 1;
+  // two temporaries before anything is touched: out of memory leaves s as it was
+  Buffer *tmp[2] = {nullptr, nullptr};
+  auto done = [&](int rc) {
+    for (Buffer *b : tmp)
+      if (b) release_buffer(b);
+    return rc;
+  };
+  for (Buffer *&b : tmp) {
+    const int rc = new_buffer(c, s->n, &b);
+    if (rc != QB_OK) return done(rc);
+  }
+  // s's shard is about to hold T_k: nobody else may see it (a clone of the old value moves to a copy)
+  int rc = make_unique(s);
+  if (rc != QB_OK) return done(rc);
+  Buffer *sb = s->b;
+  if (!(std::isfinite(sb->pscale[0]) && std::isfinite(sb->pscale[1]))) {  // NaN / inf must reach the data
+    if ((rc = force_scale(sb)) != QB_OK) return done(rc);
+  }
+  const PauliTerms h(std::move(lx), std::move(lz), std::move(cf));
+  // cur = T_{k-1}, prev = T_{k-2} (becomes T_k), acc = sum_{j < k} a_j T_j; the pending scalar rides along
+  Buffer *cur = sb, *prev = tmp[0], *acc = tmp[1];
+  for (int64_t k = 1; k <= K && rc == QB_OK; ++k) {
+    rc = run_pauli_cheb_step(cur, prev, acc, h, 1.0 / r, k, &a[0], &a[2 * k]);
+    std::swap(cur, prev);
+  }
+  if (rc != QB_OK) {
+    sb->broken = true;
+    sb->broken_why = g_last_error;
+    return done(rc);
+  }
+  // s takes acc's shard (and its peer table); tmp[1] leaves with s's old one
+  std::swap(sb->amps, acc->amps);
+  std::swap(sb->peers, acc->peers);
+  sb->perm = acc->perm;
+  const double pr = sb->pscale[0] * phase[0] - sb->pscale[1] * phase[1];
+  sb->pscale[1] = sb->pscale[0] * phase[1] + sb->pscale[1] * phase[0];
+  sb->pscale[0] = pr;
+  // every T_k(H') moves amplitude j only to j ^ (X masks of h): what s knew outside them still holds (§3.3b)
+  sb->zmask = sb->all_finite ? sb->zmask & ~xunion : 0;
+  sb->zval &= sb->zmask;
+  if (nsteps) *nsteps = K;
   return done(QB_OK);
 }
 

@@ -1357,6 +1357,22 @@ __device__ __forceinline__ void cp_async16(void *smem, const void *gmem) {
                : "memory");
 }
 
+// (H_run src)_u of tile-local index u, the tile of src in shared memory: the run's terms summed in order
+__device__ __forceinline__ void pauli_term_sum(const PauliSumArgs &a, const double2 *tile, uint32_t u, uint64_t base,
+                                               double &hr, double &hi) {
+  hr = 0.0;
+  hi = 0.0;
+  for (uint32_t i = 0; i < a.nterms; ++i) {
+    const PauliSumParam &p = a.term[i];
+    const uint32_t v = u ^ p.xt;
+    const double2 w = tile[swz(v)];
+    const bool neg = (uint32_t(__popc(v & p.zt)) ^ uint32_t(__popcll(base & p.zout))) & 1u;
+    const double cr = neg ? -p.cr : p.cr, ci = neg ? -p.ci : p.ci;
+    hr = fma(cr, w.x, fma(-ci, w.y, hr));
+    hi = fma(cr, w.y, fma(ci, w.x, hi));
+  }
+}
+
 // out (+)= H_run src over one tile per step.  The tile of src is read by every thread after one barrier; each
 // thread then sums the run's terms for its own indices without further barriers.
 template <int TB>
@@ -1367,7 +1383,7 @@ __global__ void __launch_bounds__(kPauliThreads, 3) k_pauli_sum_tile(const doubl
   static_assert(kPauliThreads == 1 << kThrBits && TB > kThrBits, "tile-local index = thread + k * kPauliThreads");
   constexpr int EPT = 1 << (TB - kThrBits);
   extern __shared__ double2 tile[];
-  const uint32_t tid = threadIdx.x, nel = 1u << a.tile_bits, nterms = a.nterms;
+  const uint32_t tid = threadIdx.x, nel = 1u << a.tile_bits;
   const PauliTileMap<TB, kThrBits> map(a, tid);
   double acc[1] = {0.0};
   for (uint64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
@@ -1381,16 +1397,8 @@ __global__ void __launch_bounds__(kPauliThreads, 3) k_pauli_sum_tile(const doubl
     for (int k = 0; k < EPT; ++k) {
       const uint32_t u = tid + k * kPauliThreads;
       if (u >= nel) continue;
-      double hr = 0.0, hi = 0.0;
-      for (uint32_t i = 0; i < nterms; ++i) {
-        const PauliSumParam &p = a.term[i];
-        const uint32_t v = u ^ p.xt;
-        const double2 w = tile[swz(v)];
-        const bool neg = (uint32_t(__popc(v & p.zt)) ^ uint32_t(__popcll(base & p.zout))) & 1u;
-        const double cr = neg ? -p.cr : p.cr, ci = neg ? -p.ci : p.ci;
-        hr = fma(cr, w.x, fma(-ci, w.y, hr));
-        hi = fma(cr, w.y, fma(ci, w.x, hi));
-      }
+      double hr, hi;
+      pauli_term_sum(a, tile, u, base, hr, hi);
       if (partials) {
         const double2 s = tile[swz(u)];
         acc[0] = fma(s.x, hr, fma(s.y, hi, acc[0]));
@@ -1406,6 +1414,56 @@ __global__ void __launch_bounds__(kPauliThreads, 3) k_pauli_sum_tile(const doubl
     __syncthreads();  // the next tile's load overwrites what other threads read
   }
   if (partials) block_reduce_store<1>(acc, partials + blockIdx.x);
+}
+
+// One launch of a Chebyshev step (qb_pauli_evolve): hs = H_run cur as in k_pauli_sum_tile, then out (the buffer
+// of T_{k-1} that becomes T_{k+1}) and, in the step's last launch, acc from the new out.  cur's tile is in shared
+// memory, so step 1's a_0 T_0 costs no extra read.
+template <int TB>
+__global__ void __launch_bounds__(kPauliThreads, 3) k_pauli_cheb_tile(const double2 *__restrict__ cur, double2 *__restrict__ out,
+                                                                     double2 *__restrict__ acc,
+                                                                     const __grid_constant__ PauliChebArgs a, uint64_t ntiles) {
+  constexpr int kThrBits = 8;
+  static_assert(kPauliThreads == 1 << kThrBits && TB > kThrBits, "tile-local index = thread + k * kPauliThreads");
+  constexpr int EPT = 1 << (TB - kThrBits);
+  extern __shared__ double2 tile[];
+  const uint32_t tid = threadIdx.x, nel = 1u << a.sum.tile_bits;
+  const PauliTileMap<TB, kThrBits> map(a.sum, tid);
+  for (uint64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
+    const uint64_t base = pauli_tile_base(a.sum, t);
+#pragma unroll
+    for (int k = 0; k < EPT; ++k)
+      if (tid + k * kPauliThreads < nel) cp_async16(tile + swz(tid + k * kPauliThreads), cur + (base | map.at(k)));
+    asm volatile("cp.async.wait_all;" ::: "memory");
+    __syncthreads();
+#pragma unroll 2
+    for (int k = 0; k < EPT; ++k) {
+      const uint32_t u = tid + k * kPauliThreads;
+      if (u >= nel) continue;
+      double hr, hi;
+      pauli_term_sum(a.sum, tile, u, base, hr, hi);
+      const uint64_t g = base | map.at(k);
+      if (a.out_mode != kChebOutStore) {
+        const double2 o = __ldcs(out + g);
+        const double sg = a.out_mode == kChebOutSub ? -1.0 : 1.0;
+        hr = fma(sg, o.x, hr);
+        hi = fma(sg, o.y, hi);
+      }
+      __stcs(out + g, make_double2(hr, hi));
+      if (a.acc_mode == kChebAccNone) continue;
+      double2 r;
+      if (a.acc_mode == kChebAccFirst) {
+        const double2 c = tile[swz(u)];
+        r = make_double2(a.a0r * c.x - a.a0i * c.y, a.a0r * c.y + a.a0i * c.x);
+      } else {
+        r = __ldcs(acc + g);
+      }
+      r.x = fma(a.akr, hr, fma(-a.aki, hi, r.x));
+      r.y = fma(a.akr, hi, fma(a.aki, hr, r.y));
+      __stcs(acc + g, r);
+    }
+    __syncthreads();  // the next tile's load overwrites what other threads read
+  }
 }
 
 // Rotations nrot-1 .. 0 undone on tiles of psi and lam, each rotation's part of Im <lam|P|psi> taken first.
@@ -1531,6 +1589,20 @@ cudaError_t launch_pauli_sum(const double2 *src, double2 *out, int local_bits, c
   if (e != cudaSuccess) return e;
   fn<<<g, kPauliThreads, sizeof(double2) << args.tile_bits, stream>>>(src, out, args, ntiles, partials_dev);
   if (partials_dev) k_expect_final<<<1, kRedThreads, 0, stream>>>(partials_dev, g, 1, energy_dev);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_pauli_cheb(const double2 *cur, double2 *out, double2 *acc, int local_bits, const PauliChebArgs &args,
+                              int sm_count, cudaStream_t stream) {
+  if (args.sum.nterms < 1 || args.sum.nterms > (uint32_t)kPauliMaxRot || args.sum.tile_bits > (uint32_t)kPauliTileBits ||
+      (int)args.sum.tile_bits > local_bits || args.out_mode > kChebOutAdd || args.acc_mode > kChebAccAdd)
+    return cudaErrorInvalidValue;
+  const auto fn = k_pauli_cheb_tile<kPauliTileBits>;
+  const uint64_t ntiles = 1ull << (local_bits - args.sum.tile_bits);
+  int g = 0;
+  cudaError_t e = pauli_walk_grid(fn, kPauliThreads, sizeof(double2) << kPauliTileBits, ntiles, sm_count, &g);
+  if (e != cudaSuccess) return e;
+  fn<<<g, kPauliThreads, sizeof(double2) << args.sum.tile_bits, stream>>>(cur, out, acc, args, ntiles);
   return cudaGetLastError();
 }
 

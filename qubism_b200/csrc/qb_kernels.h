@@ -96,6 +96,22 @@ struct PauliSumArgs {
 cudaError_t launch_pauli_sum(const double2 *src, double2 *out, int local_bits, const PauliSumArgs &args,
                              double *partials_dev, double *energy_dev, int sm_count, cudaStream_t stream);
 
+// One launch of a Chebyshev step of exp(-itH) (qb_pauli_evolve): hs = sum over the run's terms as in
+// launch_pauli_sum (the host folds 1/r, or 2/r after step 1, into the coefficients), applied to cur; then
+//   out = hs (kChebOutStore, step 1's first launch) | hs - out (kChebOutSub, a later step's first launch)
+//       | out + hs (kChebOutAdd, every other launch);
+// and in the step's last launch acc = a0 cur + ak out (kChebAccFirst, step 1) | acc + ak out (kChebAccAdd).
+// cur, out and acc are three shards in one layout.  Deterministic (fixed grid, fixed term order).
+enum : uint32_t { kChebOutStore = 0, kChebOutSub = 1, kChebOutAdd = 2 };
+enum : uint32_t { kChebAccNone = 0, kChebAccFirst = 1, kChebAccAdd = 2 };
+struct PauliChebArgs {
+  PauliSumArgs sum;  // tile geometry and terms (sum.first unused)
+  uint32_t out_mode, acc_mode;
+  double a0r, a0i, akr, aki;
+};
+cudaError_t launch_pauli_cheb(const double2 *cur, double2 *out, double2 *acc, int local_bits, const PauliChebArgs &args,
+                              int sm_count, cudaStream_t stream);
+
 // The backward pass of the adjoint gradient (qb_pauli_rot_grad) over one launch of rotations: psi and lam
 // (same layout) are walked through rotations nrot-1 .. 0; for each, grad_dev[r] = Im sum_j conj(lam_j) (P_r psi)_j,
 // then psi <- R_r^dagger psi and lam <- R_r^dagger lam with R_r^dagger = c I + i s P_r.  (P psi)_j =

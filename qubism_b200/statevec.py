@@ -362,6 +362,19 @@ class StateVec:
                                                 C.byref(energy), grad.ctypes.data_as(PD)))
         return energy.value, grad
 
+    def pauli_evolve_(self, terms, coefs, t: float):
+        """``exp(-i t H) #> self`` in place with ``H = sum_t coefs[t] P_t`` (qb_pauli_evolve: exact to double
+        precision by a Chebyshev expansion; runs at once, lazy clones keep the old value).  Terms are spelled as
+        for ``expect_pauli``; ``coefs`` are real.  Returns ``self``."""
+        xs, zs = pauli_masks(terms, self.n)
+        cf = np.ascontiguousarray(coefs, dtype=np.float64).reshape(-1)
+        if cf.size != xs.size:
+            raise ValueError(f"{xs.size} Pauli strings but {cf.size} coefficients")
+        P64 = C.POINTER(C.c_uint64)
+        capi.check(self.ctx.L.qb_pauli_evolve(self._h, xs.ctypes.data_as(P64), zs.ctypes.data_as(P64),
+                                              cf.ctypes.data_as(C.POINTER(C.c_double)), len(xs), float(t), None))
+        return self
+
     def norm(self) -> float:  # Algebra.hs:35-36: realPart (a <.> a), the SQUARED norm
         return self.inner(self).real
 
@@ -459,3 +472,9 @@ def pauliSum(terms, coefs, sv: StateVec) -> StateVec:
 def pauliRotGrad(rot_terms, thetas, h_terms, h_coefs, sv: StateVec):
     """``(energy, grad)`` of a Pauli-sum energy over Pauli rotations of ``sv`` (see StateVec.pauli_rot_grad)."""
     return sv.pauli_rot_grad(rot_terms, thetas, h_terms, h_coefs)
+
+
+def pauliEvolve(terms, coefs, t: float, sv: StateVec) -> StateVec:
+    """``exp(-i t H) #> sv`` with ``H = sum_t coefs[t] P_t`` as a new value; ``sv`` keeps its own (a lazy clone
+    evolved in place, see StateVec.pauli_evolve_)."""
+    return sv.clone().pauli_evolve_(terms, coefs, t)
