@@ -61,3 +61,5 @@ foreign import ccall safe   "qb_pauli_sum"       c_qb_pauli_sum       :: Ptr QbS
 foreign import ccall safe   "qb_pauli_rot_grad"  c_qb_pauli_rot_grad  :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Ptr CDouble -> Int64 -> Ptr Word64 -> Ptr Word64 -> Ptr CDouble -> Int64 -> Ptr CDouble -> Ptr CDouble -> IO CInt
 -- exact time evolution under Pauli sums ------------------------------------------------------
 foreign import ccall safe   "qb_pauli_evolve"    c_qb_pauli_evolve    :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Ptr CDouble -> Int64 -> CDouble -> Ptr Int64 -> IO CInt
+-- Lanczos ground states of Pauli sums ---------------------------------------------------------
+foreign import ccall safe   "qb_pauli_ground"    c_qb_pauli_ground    :: Ptr QbState -> Ptr Word64 -> Ptr Word64 -> Ptr CDouble -> Int64 -> CDouble -> Int64 -> CInt -> Ptr CDouble -> Ptr CDouble -> Ptr Int64 -> Ptr CDouble -> Ptr CDouble -> IO CInt

@@ -1,8 +1,8 @@
 {-|
 Module      : Qubism.Expect
-Description : expectation values of Pauli strings, Pauli rotations, Pauli sums, adjoint gradients and exact
-              time evolution, computed on the device (qb_expect_pauli, qb_apply_pauli_rot, qb_pauli_sum,
-              qb_pauli_rot_grad, qb_pauli_evolve)
+Description : expectation values of Pauli strings, Pauli rotations, Pauli sums, adjoint gradients, exact
+              time evolution and Lanczos ground states, computed on the device (qb_expect_pauli,
+              qb_apply_pauli_rot, qb_pauli_sum, qb_pauli_rot_grad, qb_pauli_evolve, qb_pauli_ground)
 
 @expectPauli terms sv@ is @[realPart (sv <.> (p #> sv)) | p <- terms]@ for the Pauli strings @p@ that
 @terms@ name (QGate.hs:90-108 for pauliX / pauliY / pauliZ), without building any @p #> sv@: one
@@ -20,8 +20,12 @@ run of rotations whose X qubits fit one tile together.
 one @pauliSum@ and one backward pass, whatever the number of angles).
 
 @pauliEvolve h t sv@ is @exp (-i t H) #> sv@ for @H = sum_t h_t p_t@ (real coefficients), as a new value: a
-Chebyshev expansion exact to double precision (clone + in-place evolution).  UNVERIFIED BY COMPILATION (no
-GHC in the build image).
+Chebyshev expansion exact to double precision (clone + in-place evolution).
+
+@pauliGround h tol maxiter sv@ is @(e, x)@: the lowest Lanczos Ritz value @e@ of @H = sum_t h_t p_t@ on the
+Krylov space of @sv@ (the lowest eigenvalue among the eigenvectors @sv@ overlaps), stopped once the Ritz
+residual estimate is at most @tol@ or after @maxiter@ steps, and its normalised Ritz vector @x@ as a new value
+(clone + in-place Lanczos).  UNVERIFIED BY COMPILATION (no GHC in the build image).
 -}
 {-# LANGUAGE DataKinds, KindSignatures, ScopedTypeVariables #-}
 module Qubism.Expect
@@ -31,6 +35,7 @@ module Qubism.Expect
   , pauliSum
   , pauliRotGrad
   , pauliEvolve
+  , pauliGround
   ) where
 
 import GHC.TypeLits
@@ -99,6 +104,19 @@ pauliEvolve h t sv = unsafePerformIO $ do
   withArrayLen xs $ \k px -> withArray zs $ \pz -> withArray (map realToFrac hcs) $ \pc -> withSV r $ \p -> do
     rc <- c_qb_pauli_evolve p px pz pc (fromIntegral k) (realToFrac t) nullPtr
     if rc /= 0 then error ("qubism_sv: status " ++ show rc) else pure r
+  where
+    (terms, hcs) = unzip h
+    (xs, zs) = unzip (map masks terms)
+
+-- | Real coefficients: H is Hermitian.  The same strings are errors as for pauliRotate.
+pauliGround :: KnownNat n => [([(Finite n, Pauli)], Double)] -> Double -> Int -> StateVec n -> (Double, StateVec n)
+pauliGround h tol maxiter sv = unsafePerformIO $ do
+  r <- cloneSV sv
+  withArrayLen xs $ \k px -> withArray zs $ \pz -> withArray (map realToFrac hcs) $ \pc -> withSV r $ \p ->
+    alloca $ \pe -> alloca $ \pr -> alloca $ \pm -> do
+      rc <- c_qb_pauli_ground p px pz pc (fromIntegral k) (realToFrac tol) (fromIntegral maxiter) 1 pe pr pm
+                              nullPtr nullPtr
+      if rc /= 0 then error ("qubism_sv: status " ++ show rc) else (\e -> (realToFrac e, r)) <$> peek pe
   where
     (terms, hcs) = unzip h
     (xs, zs) = unzip (map masks terms)

@@ -273,6 +273,43 @@ int qb_pauli_rot_grad(qb_state *s, const uint64_t *rx, const uint64_t *rz, const
 int qb_pauli_evolve(qb_state *s, const uint64_t *hx, const uint64_t *hz, const double *hcoef, int64_t nterms,
                     double t, int64_t *nsteps);
 
+/* ---- Lanczos ground states of Pauli sums -------------------------------------------------- */
+/* The lowest eigenvalue of H = sum_t hcoef[t] P_t (strings and real coefficients read exactly as by
+ * qb_pauli_evolve: equal strings add, zero coefficients drop out, the identity strings are a shift c) on the
+ * Krylov space of s, by plain Lanczos (no reorthogonalisation) started from s (not necessarily normalised; its
+ * pending scalar counts).  *energy = the lowest Ritz value theta of H on that space, c included: the lowest
+ * eigenvalue among the eigenvectors s overlaps -- a start state inside a symmetry sector of H gives that sector's
+ * minimum.  *resid = beta_m |y_m|, the Ritz residual estimate ||H x - theta x|| (y the unit eigenvector of the
+ * tridiagonal T_m, x the Ritz vector); *niter = m, the Krylov dimension reached.  alpha / beta (either may be
+ * null) hold maxiter doubles each: alpha_0 .. alpha_{m-1} (of H, c included) and beta_1 .. beta_m, the
+ * coefficients of T_m (for instance for continued-fraction spectra), the rest 0.
+ * Stops after the step at which resid <= tol (absolute, in the units of H), or beta_m <= 2^-40 r with r = sum |h|
+ * over the merged non-identity strings (an invariant subspace: |0...0> under a Heisenberg chain stops at m = 1
+ * with beta exactly 0), or m = maxiter -- not an error: QB_OK with *resid > tol, the caller decides.
+ * vector = 0: s keeps its value and its handle (also with option "linear" = 1); it is only observed (flushed).
+ * vector = 1: s becomes the normalised Ritz vector x = sum_k y_k v_k, phased so that <s_old|x> is real and
+ * positive (y_0 > 0); it changes in place as in qb_pauli_evolve (lazy clones keep the old value, option
+ * "linear" = 1 consumes them) and knows the qubits of known value that s knew outside every non-identity X mask.
+ * No non-identity string: *energy = c, m = 0, *resid = 0 (and with vector = 1 s becomes s / ||s||, deferred).
+ * Deterministic: fixed-order reductions; x is built by a second run of the same recurrence, which reproduces
+ * every v_k.  Distributed: a collective; every rank receives the same results.
+ * Cost: one norm sweep of s, then per step one launch per run of the cut qb_pauli_sum makes for the merged
+ * non-identity strings (reading v_k and v_{k-1}, writing w; the last also reduces alpha) and one update sweep
+ * (48 B per amplitude: w -= alpha v and ||w||^2): simple_launches grows by those launches + 1 and
+ * reduce_launches by 2 per step, besides the 2 of each norm sweep.  vector = 1 runs the recurrence twice: m - 1
+ * further steps without reductions, whose update sweeps also add to s (80 B per amplitude), and one more norm
+ * sweep.  Memory: two temporary states besides s.
+ * Everything is checked before anything is queued, allocated or written (a rejected call leaves s and its
+ * queue untouched):
+ * QB_ERR_ARG: a null s, energy, resid or niter, or a null mask / coefficient array with nterms > 0; nterms < 0; a
+ * mask bit at or above n; a non-finite coefficient; tol NaN or negative; maxiter < 1 or > QB_GROUND_MAX_ITER; a
+ * start vector of zero or non-finite norm (found by the first norm sweep, before anything is written).
+ * QB_ERR_UNSUPPORTED and QB_ERR_OOM: as for qb_pauli_evolve. */
+#define QB_GROUND_MAX_ITER 65536
+int qb_pauli_ground(qb_state *s, const uint64_t *hx, const uint64_t *hz, const double *hcoef, int64_t nterms,
+                    double tol, int64_t maxiter, int vector, double *energy, double *resid, int64_t *niter,
+                    double *alpha, double *beta);
+
 /* ---- introspection (tests, bench, profiling) ------------------------------------------- */
 typedef struct {
   uint64_t ops_submitted;   /* primitive ops received through the ABI                     */

@@ -96,6 +96,8 @@ SIGNATURES = {
     "qb_pauli_rot_grad": (_I, [_VP, C.POINTER(_U64), C.POINTER(_U64), C.POINTER(_D), _I64, C.POINTER(_U64),
                                C.POINTER(_U64), C.POINTER(_D), _I64, C.POINTER(_D), C.POINTER(_D)]),
     "qb_pauli_evolve": (_I, [_VP, C.POINTER(_U64), C.POINTER(_U64), C.POINTER(_D), _I64, _D, C.POINTER(_I64)]),
+    "qb_pauli_ground": (_I, [_VP, C.POINTER(_U64), C.POINTER(_U64), C.POINTER(_D), _I64, _D, _I64, _I, C.POINTER(_D),
+                             C.POINTER(_D), C.POINTER(_I64), C.POINTER(_D), C.POINTER(_D)]),
     "qb_get_stats": (_I, [_VP, C.POINTER(QbStats)]),
     "qb_reset_stats": (_I, [_VP]),
     "qb_ctx_stream": (_VP, [_VP]),

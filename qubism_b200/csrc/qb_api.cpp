@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cfloat>
 #include <chrono>
 #include <cmath>
 #include <cstdarg>
@@ -1510,34 +1511,87 @@ int run_pauli_sum(Buffer *src, Buffer *out, const std::vector<uint64_t> &lx, con
   return QB_OK;
 }
 
-// Step k >= 1 of the Chebyshev recurrence of qb_pauli_evolve, one launch per run of the cut of h (H' = f h with
-// f = 1 / r; the terms are scaled by f at step 1 and by 2 f later): prev <- H' cur (step 1) or 2 H' cur - prev,
-// then acc <- a0 cur + ak prev (step 1) or acc + ak prev.  All three shards end in cur's layout; prev's and
-// acc's old contents do not matter at step 1 (their first write is a store).
-int run_pauli_cheb_step(Buffer *cur, Buffer *prev, Buffer *acc, const PauliTerms &h, double f, int64_t step,
-                        const double a0[2], const double ak[2]) {
+// One step of a three-buffer recurrence, one launch per run of the cut of h with its terms scaled by f:
+// prev <- f h cur (first) or f h cur + sub prev (sub = -1 unless lz), then, when acc is given, acc <- a0 cur + ak prev
+// (first) or acc + ak prev.  Chebyshev step k of qb_pauli_evolve: f = 1 / r at step 1, 2 / r later.  lz (a Lanczos
+// step of qb_pauli_ground) carries sub, and with dot_dev, *dot_dev = Re <cur|prev> over the new prev.  All three
+// shards end in cur's layout; prev's and acc's old contents do not matter at the first step (their first write is
+// a store).
+int run_pauli_cheb_step(Buffer *cur, Buffer *prev, Buffer *acc, const PauliTerms &h, double f, bool first,
+                        const double a0[2], const double ak[2], const PauliLanczosArgs *lz = nullptr) {
   qb_ctx *c = cur->ctx;
   for (size_t i0 = 0, i1 = 0; i0 < h.sx.size(); i0 = i1) {
     PauliChebArgs args;
-    QB_TRY(pauli_sum_launch(cur, h, step == 1 ? f : 2.0 * f, i0, &i1, args.sum));
-    const bool first = i0 == 0, last = i1 == h.sx.size();
-    if (step == 1 && first) prev->perm = cur->perm;
+    QB_TRY(pauli_sum_launch(cur, h, f, i0, &i1, args.sum));
+    const bool head = i0 == 0, last = i1 == h.sx.size();
+    if (first && head) prev->perm = cur->perm;
     else if (prev->perm != cur->perm) QB_TRY(relayout(prev, cur->perm));
-    if (step == 1) {
-      if (last) acc->perm = cur->perm;  // (acc is first written, whole, by step 1's last launch)
-    } else if (acc->perm != cur->perm) {
+    if (acc && first) {
+      if (last) acc->perm = cur->perm;  // (acc is first written, whole, by the first step's last launch)
+    } else if (acc && acc->perm != cur->perm) {
       QB_TRY(relayout(acc, cur->perm));
     }
-    args.out_mode = !first ? kChebOutAdd : step == 1 ? kChebOutStore : kChebOutSub;
-    args.acc_mode = !last ? kChebAccNone : step == 1 ? kChebAccFirst : kChebAccAdd;
+    args.out_mode = !head ? kChebOutAdd : first ? kChebOutStore : kChebOutSub;
+    args.acc_mode = !acc || !last ? kChebAccNone : first ? kChebAccFirst : kChebAccAdd;
     args.a0r = a0[0];
     args.a0i = a0[1];
     args.akr = ak[0];
     args.aki = ak[1];
-    QB_CUDA(launch_pauli_cheb(cur->amps, prev->amps, acc->amps, cur->L, args, c->sm_count, c->stream));
+    PauliLanczosArgs l{};
+    if (lz) {
+      l = *lz;
+      if (!last) l.partials_dev = l.dot_dev = nullptr;
+    }
+    QB_CUDA(launch_pauli_cheb(cur->amps, prev->amps, acc ? acc->amps : nullptr, cur->L, args, c->sm_count, c->stream,
+                              lz ? &l : nullptr));
     c->stats.simple_launches++;
+    if (l.dot_dev) c->stats.reduce_launches++;
   }
   return QB_OK;
+}
+
+// A real Pauli sum H = cid I + sum_k cf[2k] P_k from the caller's strings: equal strings added (first appearance
+// order), zero sums dropped, the identity strings apart in cid.  Logical masks; cf holds (re, 0) pairs as
+// PauliTerms wants them; r = sum |cf| and xunion = the union of the X masks, both over the kept strings.
+struct RealPauliSum {
+  double cid = 0.0, r = 0.0;
+  uint64_t xunion = 0;
+  std::vector<uint64_t> lx, lz;
+  std::vector<double> cf;
+};
+
+RealPauliSum merge_pauli_sum(int n, const uint64_t *hx, const uint64_t *hz, const double *hcoef, int64_t nterms) {
+  RealPauliSum m;
+  std::map<std::pair<uint64_t, uint64_t>, size_t> seen;
+  for (int64_t k = 0; k < nterms; ++k) {
+    if (!(hx[k] | hz[k])) {
+      m.cid += hcoef[k];
+      continue;
+    }
+    const auto it = seen.emplace(std::make_pair(hx[k], hz[k]), m.lx.size());
+    if (it.second) {
+      m.lx.push_back(logical_mask(n, hx[k]));
+      m.lz.push_back(logical_mask(n, hz[k]));
+      m.cf.push_back(hcoef[k]);
+      m.cf.push_back(0.0);
+    } else {
+      m.cf[2 * it.first->second] += hcoef[k];
+    }
+  }
+  size_t nh = 0;
+  for (size_t k = 0; k < m.lx.size(); ++k) {
+    if (m.cf[2 * k] == 0.0) continue;
+    m.r += std::fabs(m.cf[2 * k]);
+    m.xunion |= m.lx[k];
+    m.lx[nh] = m.lx[k];
+    m.lz[nh] = m.lz[k];
+    m.cf[2 * nh] = m.cf[2 * k];
+    ++nh;
+  }
+  m.lx.resize(nh);
+  m.lz.resize(nh);
+  m.cf.resize(2 * nh);
+  return m;
 }
 
 // The Chebyshev coefficients of exp(-i tau x) on [-1, 1]: a[k] = (re, im) of a_0 = J_0(tau), a_k = 2 (-i)^k J_k(tau)
@@ -2476,39 +2530,9 @@ int qb_pauli_evolve(qb_state *s, const uint64_t *hx, const uint64_t *hz, const d
   QB_TRY(check_state(s));
   if (t == 0.0 || nterms == 0) return QB_OK;
   // H = cid I + h: equal strings merged (caller order), zero coefficients dropped, the identity apart
-  double cid = 0.0, r = 0.0;
-  std::vector<uint64_t> lx, lz;
-  std::vector<double> cf;
-  std::map<std::pair<uint64_t, uint64_t>, size_t> seen;
-  for (int64_t k = 0; k < nterms; ++k) {
-    if (!(hx[k] | hz[k])) {
-      cid += hcoef[k];
-      continue;
-    }
-    const auto it = seen.emplace(std::make_pair(hx[k], hz[k]), lx.size());
-    if (it.second) {
-      lx.push_back(logical_mask(s->n, hx[k]));
-      lz.push_back(logical_mask(s->n, hz[k]));
-      cf.push_back(hcoef[k]);
-      cf.push_back(0.0);
-    } else {
-      cf[2 * it.first->second] += hcoef[k];
-    }
-  }
-  uint64_t xunion = 0;
-  size_t nh = 0;
-  for (size_t k = 0; k < lx.size(); ++k) {
-    if (cf[2 * k] == 0.0) continue;
-    r += std::fabs(cf[2 * k]);
-    xunion |= lx[k];
-    lx[nh] = lx[k];
-    lz[nh] = lz[k];
-    cf[2 * nh] = cf[2 * k];
-    ++nh;
-  }
-  lx.resize(nh);
-  lz.resize(nh);
-  cf.resize(2 * nh);
+  RealPauliSum m = merge_pauli_sum(s->n, hx, hz, hcoef, nterms);
+  const double cid = m.cid, r = m.r;
+  const uint64_t xunion = m.xunion;
   const double tc = t * cid;
   if (!std::isfinite(tc)) return fail(QB_ERR_ARG, "t times the identity coefficient is not finite");
   const double phase[2] = {std::cos(tc), -std::sin(tc)};  // e^{-itc}
@@ -2544,11 +2568,12 @@ int qb_pauli_evolve(qb_state *s, const uint64_t *hx, const uint64_t *hz, const d
   if (!(std::isfinite(sb->pscale[0]) && std::isfinite(sb->pscale[1]))) {  // NaN / inf must reach the data
     if ((rc = force_scale(sb)) != QB_OK) return done(rc);
   }
-  const PauliTerms h(std::move(lx), std::move(lz), std::move(cf));
+  const PauliTerms h(std::move(m.lx), std::move(m.lz), std::move(m.cf));
   // cur = T_{k-1}, prev = T_{k-2} (becomes T_k), acc = sum_{j < k} a_j T_j; the pending scalar rides along
   Buffer *cur = sb, *prev = tmp[0], *acc = tmp[1];
+  const double f = 1.0 / r;
   for (int64_t k = 1; k <= K && rc == QB_OK; ++k) {
-    rc = run_pauli_cheb_step(cur, prev, acc, h, 1.0 / r, k, &a[0], &a[2 * k]);
+    rc = run_pauli_cheb_step(cur, prev, acc, h, k == 1 ? f : 2.0 * f, k == 1, &a[0], &a[2 * k]);
     std::swap(cur, prev);
   }
   if (rc != QB_OK) {
@@ -2567,6 +2592,271 @@ int qb_pauli_evolve(qb_state *s, const uint64_t *hx, const uint64_t *hz, const d
   sb->zmask = sb->all_finite ? sb->zmask & ~xunion : 0;
   sb->zval &= sb->zmask;
   if (nsteps) *nsteps = K;
+  return done(QB_OK);
+}
+
+// ---- Lanczos ground states of Pauli sums
+// The lowest eigenvalue theta of the symmetric tridiagonal T_m (diagonal al[0..m), off-diagonal be[0..m-1): be[i]
+// couples rows i and i + 1) and its unit eigenvector y with y[0] >= 0.  Deterministic and O(m): Sturm-sequence
+// bisection from the Gershgorin interval to the last bit, then two inverse-iteration solves with (T - theta I)
+// factored by Gaussian elimination with partial pivoting (pivots below eps ||T|| replaced by that).
+static double tridiag_lowest(const double *al, const double *be, int64_t m, std::vector<double> &y) {
+  if (m == 1) {
+    y.assign(1, 1.0);
+    return al[0];
+  }
+  double bmax2 = 0.0, gl = al[0], gu = al[0];
+  for (int64_t i = 0; i < m; ++i) {
+    const double rad = (i > 0 ? std::fabs(be[i - 1]) : 0.0) + (i + 1 < m ? std::fabs(be[i]) : 0.0);
+    gl = std::min(gl, al[i] - rad);
+    gu = std::max(gu, al[i] + rad);
+    if (i + 1 < m) bmax2 = std::max(bmax2, be[i] * be[i]);
+  }
+  const double eps = 0x1p-53, pivmin = DBL_MIN * std::max(1.0, bmax2);
+  const double tnorm = std::max(std::fabs(gl), std::fabs(gu));
+  const double pad = 2.0 * eps * tnorm * double(m) + 2.0 * pivmin;
+  auto below = [&](double x) {  // the number of eigenvalues below x (Sturm count from the LDL^T pivots)
+    int64_t cnt = 0;
+    double d = 1.0;
+    for (int64_t i = 0; i < m; ++i) {
+      d = al[i] - x - (i > 0 ? be[i - 1] * be[i - 1] / d : 0.0);
+      if (std::fabs(d) < pivmin) d = -pivmin;
+      if (d < 0.0) ++cnt;
+    }
+    return cnt;
+  };
+  double lo = gl - pad, hi = gu + pad;  // below(lo) = 0 <= 1 <= below(hi)
+  for (int it = 0; it < 256; ++it) {
+    const double mid = 0.5 * (lo + hi);
+    if (mid <= lo || mid >= hi || hi - lo <= 2.0 * eps * std::max(std::fabs(lo), std::fabs(hi)) + pivmin) break;
+    if (below(mid) >= 1) hi = mid;
+    else lo = mid;
+  }
+  const double theta = 0.5 * (lo + hi);
+  // (T - theta I) = P L U: d the diagonal, du / du2 the first / second super-diagonals of U, dl the multipliers
+  std::vector<double> d(m), du(m, 0.0), du2(m, 0.0), dl(m, 0.0);
+  std::vector<char> swapped(m, 0);
+  for (int64_t i = 0; i < m; ++i) d[i] = al[i] - theta;
+  for (int64_t i = 0; i + 1 < m; ++i) du[i] = be[i];
+  for (int64_t i = 0; i + 1 < m; ++i) {
+    const double sub = be[i];
+    if (std::fabs(d[i]) >= std::fabs(sub)) {
+      if (d[i] != 0.0) {
+        dl[i] = sub / d[i];
+        d[i + 1] -= dl[i] * du[i];
+      }
+    } else {
+      const double fct = d[i] / sub;
+      d[i] = sub;
+      dl[i] = fct;
+      const double tmp = du[i];
+      du[i] = d[i + 1];
+      d[i + 1] = tmp - fct * d[i + 1];
+      if (i + 2 < m) {
+        du2[i] = du[i + 1];
+        du[i + 1] = -fct * du[i + 1];
+      }
+      swapped[i] = 1;
+    }
+  }
+  const double tiny = std::max(eps * tnorm, pivmin);
+  for (double &v : d)
+    if (std::fabs(v) < tiny) v = v < 0.0 ? -tiny : tiny;
+  y.assign(m, 0.0);
+  for (int64_t i = 0; i < m; ++i) y[i] = 1.0 + 0.25 * double((i * 7) % 5);  // (any start not orthogonal to the answer)
+  for (int pass = 0; pass < 2; ++pass) {
+    for (int64_t i = 0; i + 1 < m; ++i) {
+      if (swapped[i]) std::swap(y[i], y[i + 1]);
+      y[i + 1] -= dl[i] * y[i];
+    }
+    for (int64_t i = m - 1; i >= 0; --i) {
+      double v = y[i];
+      if (i + 1 < m) v -= du[i] * y[i + 1];
+      if (i + 2 < m) v -= du2[i] * y[i + 2];
+      y[i] = v / d[i];
+    }
+    double nn = 0.0, big = 0.0;
+    for (double v : y) big = std::max(big, std::fabs(v));
+    for (double &v : y) {
+      v /= big;
+      nn += v * v;
+    }
+    const double sc = (y[0] < 0.0 ? -1.0 : 1.0) / std::sqrt(nn);
+    for (double &v : y) v *= sc;
+  }
+  return theta;
+}
+
+// The Lanczos recurrence of qb_pauli_ground, plain (no reorthogonalisation) in Paige's A(2,7) form on H' = H - cid:
+//   w = H' v_k - beta_k v_{k-1},  alpha_k = Re <v_k|w>,  w -= alpha_k v_k,  beta_{k+1} = ||w||,  v_{k+1} = w / beta_{k+1}.
+// Normalisation is deferred, so every buffer holds a known positive multiple of its Lanczos vector (the phase of s's
+// pending scalar is common to every vector and stays out of the recurrence):
+//   s holds s_dev, v_0 = s_dev / ||s_dev||;  step 0's last launch also writes v_0 itself into T2 (kChebAccFirst);
+//   the buffer step k writes holds w itself, first before and then after the update, so v_{k+1} = it / beta_{k+1}.
+// Hence step k scales h by f_k = 1 / ||s_dev|| (k = 0) or 1 / beta_k, puts sub_k = -beta_k (k = 1: T2 holds v_0
+// itself) or -beta_k / beta_{k-1} on the buffer of v_{k-1}, finds alpha_k = f_k Re <cur|w>, and the update
+// subtracts alpha_k T2 (k = 0) or alpha_k f_k cur.  The buffers: step 0 reads s and writes T1 and T2; from step 1 on
+// w overwrites the buffer of v_{k-1} in place, T1 and T2 trading roles, so s is never written.  The run that builds
+// the Ritz vector x = sum_k y_k v_k repeats steps 0 .. m-2 with the stored alpha and beta (the same launches on the
+// same data: the same v_k, bit for bit, on one GPU) and, in place of the norm, accumulates x into s:
+// s <- (y_0 f_0) s + (y_1 / beta_1) w at step 0 and s <- s + (y_{k+1} / beta_{k+1}) w later.
+struct LanczosRun {
+  Buffer *s, *t1, *t2;
+  const PauliTerms &h;
+  double f0;  // 1 / ||s_dev||
+};
+
+// Step k: cur holds the multiple 1 / f of v_k, prev that of v_{k-1} (unused at k = 0).  reduce: *alpha = alpha_k
+// and *beta2 = beta_{k+1}^2 (all-reduced); otherwise alpha_k is given and s <- p s + q w.
+static int lanczos_step(const LanczosRun &L, Buffer *cur, Buffer *prev, int64_t k, double f, double sub, bool reduce,
+                 double *alpha, double *beta2, double p, double q) {
+  qb_ctx *c = cur->ctx;
+  const double zero[2] = {0.0, 0.0}, a0[2] = {f, 0.0};
+  PauliLanczosArgs lz{sub, reduce ? c->red_partials : nullptr, reduce ? c->red_out : nullptr};
+  QB_TRY(run_pauli_cheb_step(cur, prev, k == 0 ? L.t2 : nullptr, L.h, f, k == 0, a0, zero, &lz));
+  auto read_back = [&](double *v) -> int {
+    QB_CUDA(cudaMemcpyAsync(c->red_host, c->red_out, sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+    QB_CUDA(cudaStreamSynchronize(c->stream));
+    *v = c->red_host[0];
+    if (c->nranks > 1) {
+      const int rc = dist_allreduce_sum(c->dist, v, 1, c->stream);
+      if (rc != QB_OK) return fail(rc, "allreduce failed: %s", dist_last_error());
+    }
+    return QB_OK;
+  };
+  if (reduce) {
+    double dot = 0.0;
+    QB_TRY(read_back(&dot));
+    *alpha = f * dot;
+  }
+  Buffer *v = k == 0 ? L.t2 : cur, *acc = reduce ? nullptr : L.s;
+  if (acc && acc->perm != cur->perm) QB_TRY(relayout(acc, cur->perm));
+  QB_CUDA(launch_lanczos_update(prev->amps, v->amps, acc ? acc->amps : nullptr, 1ull << cur->L,
+                                k == 0 ? *alpha : *alpha * f, p, q, c->red_partials, c->red_out, c->sm_count, c->stream));
+  c->stats.simple_launches++;
+  if (reduce) {
+    c->stats.reduce_launches++;
+    QB_TRY(read_back(beta2));
+  }
+  return QB_OK;
+}
+
+// Steps 0 .. nsteps-1: the energy run (reduce; al / be filled, stopping by the rule of qb_pauli_ground, *m = the
+// Krylov dimension reached, y its Ritz vector) or the vector run (al, be and y given; nsteps = m - 1).
+static int lanczos_run(const LanczosRun &L, bool reduce, int64_t maxiter, double tol, double r, std::vector<double> &al,
+                std::vector<double> &be, std::vector<double> &y, int64_t *m, double *theta, double *resid) {
+  Buffer *cur = L.s, *prev = L.t1;
+  const int64_t nsteps = reduce ? maxiter : *m - 1;
+  for (int64_t k = 0; k < nsteps; ++k) {
+    const double f = k == 0 ? L.f0 : 1.0 / be[k - 1];
+    const double sub = k == 0 ? 0.0 : k == 1 ? -be[0] : -be[k - 1] / be[k - 2];
+    double alpha = reduce ? 0.0 : al[k], beta2 = 0.0;
+    const double p = !reduce && k == 0 ? y[0] * L.f0 : 1.0, q = reduce ? 0.0 : y[k + 1] / be[k];
+    QB_TRY(lanczos_step(L, cur, prev, k, f, sub, reduce, &alpha, &beta2, p, q));
+    if (k == 0) {
+      cur = L.t1;
+      prev = L.t2;
+    } else {
+      std::swap(cur, prev);
+    }
+    if (!reduce) continue;
+    al.push_back(alpha);
+    be.push_back(std::sqrt(beta2));
+    if (!std::isfinite(alpha) || !std::isfinite(be.back()))
+      return fail(QB_ERR_ARG, "Lanczos step %lld overflows: H is too large for double precision", (long long)k);
+    *theta = tridiag_lowest(al.data(), be.data(), k + 1, y);
+    *resid = be.back() * std::fabs(y.back());
+    *m = k + 1;
+    if (*resid <= tol || be.back() <= 0x1p-40 * r) break;
+  }
+  return QB_OK;
+}
+
+int qb_pauli_ground(qb_state *s, const uint64_t *hx, const uint64_t *hz, const double *hcoef, int64_t nterms, double tol,
+                    int64_t maxiter, int vector, double *energy, double *resid, int64_t *niter, double *alpha,
+                    double *beta) {
+  if (!s || !energy || !resid || !niter) return fail(QB_ERR_ARG, "null argument");
+  if (nterms < 0) return fail(QB_ERR_ARG, "nterms %lld < 0", (long long)nterms);
+  if (nterms > 0 && (!hx || !hz || !hcoef)) return fail(QB_ERR_ARG, "null argument");
+  if (!(tol >= 0.0)) return fail(QB_ERR_ARG, "tol is NaN or negative");
+  if (maxiter < 1 || maxiter > QB_GROUND_MAX_ITER)
+    return fail(QB_ERR_ARG, "maxiter %lld outside 1 .. %d", (long long)maxiter, QB_GROUND_MAX_ITER);
+  QB_TRY(check_pauli_strings(s, "term", "coefficient", hx, hz, hcoef, 1, nterms));
+  qb_ctx *c = s->ctx;
+  Guard g(c);
+  QB_TRY(check_state(s));
+  RealPauliSum hm = merge_pauli_sum(s->n, hx, hz, hcoef, nterms);
+  if (!std::isfinite(hm.r) || !std::isfinite(hm.cid)) return fail(QB_ERR_ARG, "sum |h| is not finite");
+  // the start vector: observed, and its norm found before anything is allocated or written
+  QB_TRY(materialise(s));
+  Buffer *sb = s->b;
+  QB_TRY(ensure_inplace(sb));
+  const double ps[2] = {sb->pscale[0], sb->pscale[1]};
+  const double pabs = std::hypot(ps[0], ps[1]);
+  double nrm2 = 0.0;
+  if (std::isfinite(pabs)) QB_TRY(sumsq_buffer(sb, -1, &nrm2, nullptr));  // (|pscale|^2 ||s_dev||^2)
+  if (!(std::isfinite(pabs) && std::isfinite(nrm2) && nrm2 > 0.0 && pabs > 0.0))
+    return fail(QB_ERR_ARG, "the start vector has norm %g", std::sqrt(nrm2));
+  const double snorm = std::sqrt(nrm2), f0 = pabs / snorm;  // f0 = 1 / ||s_dev||
+  auto outputs = [&](double e, double res, int64_t m, const std::vector<double> &al, const std::vector<double> &be) {
+    *energy = e;
+    *resid = res;
+    *niter = m;
+    for (int64_t k = 0; k < maxiter; ++k) {
+      if (alpha) alpha[k] = k < m ? al[k] + hm.cid : 0.0;
+      if (beta) beta[k] = k < m ? be[k] : 0.0;
+    }
+  };
+  if (hm.r == 0.0) {  // H = cid I: every vector is an eigenvector
+    outputs(hm.cid, 0.0, 0, {}, {});
+    if (!vector) return QB_OK;
+    LogOp o;
+    o.kind = LOG_SCALE;
+    o.m[0] = 1.0 / snorm;
+    return append(s, std::move(o));
+  }
+  // two temporaries before anything is touched: out of memory leaves s as it was
+  Buffer *tmp[2] = {nullptr, nullptr};
+  auto done = [&](int rc) {
+    for (Buffer *b : tmp)
+      if (b) release_buffer(b);
+    return rc;
+  };
+  for (Buffer *&b : tmp) {
+    const int rc = new_buffer(c, s->n, &b);
+    if (rc != QB_OK) return done(rc);
+  }
+  int rc = QB_OK;
+  if (vector) {  // s's shard will hold x: nobody else may see it (a clone of the old value moves to a copy)
+    if ((rc = make_unique(s)) != QB_OK) return done(rc);
+    sb = s->b;
+  }
+  const PauliTerms h(std::move(hm.lx), std::move(hm.lz), std::move(hm.cf));
+  const LanczosRun L{sb, tmp[0], tmp[1], h, f0};
+  std::vector<double> al, be, y;
+  int64_t m = 0;
+  double theta = 0.0, res = 0.0;
+  rc = lanczos_run(L, true, maxiter, tol, hm.r, al, be, y, &m, &theta, &res);
+  if (rc == QB_OK && vector) rc = lanczos_run(L, false, maxiter, tol, hm.r, al, be, y, &m, &theta, &res);
+  if (rc != QB_OK) {
+    if (vector) {
+      sb->broken = true;
+      sb->broken_why = g_last_error;
+    }
+    return done(rc);
+  }
+  if (vector) {  // s holds a positive multiple of x: its norm and the old scalar's phase go to the pending scalar
+    sb->zmask = sb->all_finite ? sb->zmask & ~hm.xunion : 0;  // (every v_k moves amplitude j only to j ^ X masks)
+    sb->zval &= sb->zmask;
+    sb->pscale[0] = 1.0;
+    sb->pscale[1] = 0.0;
+    double xn2 = 0.0;
+    if ((rc = sumsq_buffer(sb, -1, &xn2, nullptr)) != QB_OK) return done(rc);
+    const double xs = 1.0 / (std::sqrt(xn2) * pabs);
+    sb->pscale[0] = ps[0] * xs;
+    sb->pscale[1] = ps[1] * xs;
+  }
+  outputs(theta + hm.cid, res, m, al, be);
   return done(QB_OK);
 }
 

@@ -1419,16 +1419,20 @@ __global__ void __launch_bounds__(kPauliThreads, 3) k_pauli_sum_tile(const doubl
 // One launch of a Chebyshev step (qb_pauli_evolve): hs = H_run cur as in k_pauli_sum_tile, then out (the buffer
 // of T_{k-1} that becomes T_{k+1}) and, in the step's last launch, acc from the new out.  cur's tile is in shared
 // memory, so step 1's a_0 T_0 costs no extra read.
-template <int TB>
+// LZ, a Lanczos step (qb_pauli_ground): Sub mode puts osub, not -1, on the old out, and with partials (the step's
+// last launch) each block leaves its share of Re <cur|out> over the new out, read from the tile in shared memory.
+template <int TB, bool LZ>
 __global__ void __launch_bounds__(kPauliThreads, 3) k_pauli_cheb_tile(const double2 *__restrict__ cur, double2 *__restrict__ out,
                                                                      double2 *__restrict__ acc,
-                                                                     const __grid_constant__ PauliChebArgs a, uint64_t ntiles) {
+                                                                     const __grid_constant__ PauliChebArgs a, uint64_t ntiles,
+                                                                     double *__restrict__ partials, double osub) {
   constexpr int kThrBits = 8;
   static_assert(kPauliThreads == 1 << kThrBits && TB > kThrBits, "tile-local index = thread + k * kPauliThreads");
   constexpr int EPT = 1 << (TB - kThrBits);
   extern __shared__ double2 tile[];
   const uint32_t tid = threadIdx.x, nel = 1u << a.sum.tile_bits;
   const PauliTileMap<TB, kThrBits> map(a.sum, tid);
+  double dot[1] = {0.0};
   for (uint64_t t = blockIdx.x; t < ntiles; t += gridDim.x) {
     const uint64_t base = pauli_tile_base(a.sum, t);
 #pragma unroll
@@ -1445,11 +1449,15 @@ __global__ void __launch_bounds__(kPauliThreads, 3) k_pauli_cheb_tile(const doub
       const uint64_t g = base | map.at(k);
       if (a.out_mode != kChebOutStore) {
         const double2 o = __ldcs(out + g);
-        const double sg = a.out_mode == kChebOutSub ? -1.0 : 1.0;
+        const double sg = a.out_mode == kChebOutSub ? (LZ ? osub : -1.0) : 1.0;
         hr = fma(sg, o.x, hr);
         hi = fma(sg, o.y, hi);
       }
       __stcs(out + g, make_double2(hr, hi));
+      if (LZ && partials) {
+        const double2 c = tile[swz(u)];
+        dot[0] = fma(c.x, hr, fma(c.y, hi, dot[0]));
+      }
       if (a.acc_mode == kChebAccNone) continue;
       double2 r;
       if (a.acc_mode == kChebAccFirst) {
@@ -1464,6 +1472,7 @@ __global__ void __launch_bounds__(kPauliThreads, 3) k_pauli_cheb_tile(const doub
     }
     __syncthreads();  // the next tile's load overwrites what other threads read
   }
+  if (LZ && partials) block_reduce_store<1>(dot, partials + blockIdx.x);
 }
 
 // Rotations nrot-1 .. 0 undone on tiles of psi and lam, each rotation's part of Im <lam|P|psi> taken first.
@@ -1593,16 +1602,55 @@ cudaError_t launch_pauli_sum(const double2 *src, double2 *out, int local_bits, c
 }
 
 cudaError_t launch_pauli_cheb(const double2 *cur, double2 *out, double2 *acc, int local_bits, const PauliChebArgs &args,
-                              int sm_count, cudaStream_t stream) {
+                              int sm_count, cudaStream_t stream, const PauliLanczosArgs *lz) {
   if (args.sum.nterms < 1 || args.sum.nterms > (uint32_t)kPauliMaxRot || args.sum.tile_bits > (uint32_t)kPauliTileBits ||
-      (int)args.sum.tile_bits > local_bits || args.out_mode > kChebOutAdd || args.acc_mode > kChebAccAdd)
+      (int)args.sum.tile_bits > local_bits || args.out_mode > kChebOutAdd || args.acc_mode > kChebAccAdd ||
+      (lz && lz->partials_dev && !lz->dot_dev))
     return cudaErrorInvalidValue;
-  const auto fn = k_pauli_cheb_tile<kPauliTileBits>;
+  const auto fn = lz ? k_pauli_cheb_tile<kPauliTileBits, true> : k_pauli_cheb_tile<kPauliTileBits, false>;
   const uint64_t ntiles = 1ull << (local_bits - args.sum.tile_bits);
   int g = 0;
   cudaError_t e = pauli_walk_grid(fn, kPauliThreads, sizeof(double2) << kPauliTileBits, ntiles, sm_count, &g);
   if (e != cudaSuccess) return e;
-  fn<<<g, kPauliThreads, sizeof(double2) << args.sum.tile_bits, stream>>>(cur, out, acc, args, ntiles);
+  double *partials = lz ? lz->partials_dev : nullptr;
+  fn<<<g, kPauliThreads, sizeof(double2) << args.sum.tile_bits, stream>>>(cur, out, acc, args, ntiles, partials,
+                                                                         lz ? lz->osub : -1.0);
+  if (partials) k_expect_final<<<1, kRedThreads, 0, stream>>>(partials, g, 1, lz->dot_dev);
+  return cudaGetLastError();
+}
+
+// One sweep of a Lanczos step (qb_pauli_ground): w <- w - a v, then either each block's share of ||w||^2 (acc null)
+// or acc <- p acc + q w (the run that builds the Ritz vector).  Fixed grid, grid-stride in a fixed order: the
+// new w is the same in both runs and the sum is deterministic.
+__global__ void __launch_bounds__(kRedThreads) k_lanczos_update(double2 *__restrict__ w, const double2 *__restrict__ v,
+                                                               double2 *__restrict__ acc, uint64_t n, double a, double p,
+                                                               double q, double *__restrict__ partials) {
+  double s[1] = {0.0};
+  const uint64_t stride = uint64_t(gridDim.x) * blockDim.x;
+  for (uint64_t i = blockIdx.x * uint64_t(blockDim.x) + threadIdx.x; i < n; i += stride) {
+    const double2 x = __ldcs(v + i);
+    double2 y = __ldcs(w + i);
+    y.x = fma(-a, x.x, y.x);
+    y.y = fma(-a, x.y, y.y);
+    __stcs(w + i, y);
+    if (acc) {
+      double2 z = __ldcs(acc + i);
+      z.x = fma(q, y.x, p * z.x);
+      z.y = fma(q, y.y, p * z.y);
+      __stcs(acc + i, z);
+    } else {
+      s[0] = fma(y.x, y.x, fma(y.y, y.y, s[0]));
+    }
+  }
+  if (!acc) block_reduce_store<1>(s, partials + blockIdx.x);
+}
+
+cudaError_t launch_lanczos_update(double2 *w, const double2 *v, double2 *acc, uint64_t n, double a, double p, double q,
+                                  double *partials_dev, double *sumsq_dev, int sm_count, cudaStream_t stream) {
+  if (!acc && !(partials_dev && sumsq_dev)) return cudaErrorInvalidValue;
+  const int g = reduce_grid(n, sm_count);
+  k_lanczos_update<<<g, kRedThreads, 0, stream>>>(w, v, acc, n, a, p, q, partials_dev);
+  if (!acc) k_expect_final<<<1, kRedThreads, 0, stream>>>(partials_dev, g, 1, sumsq_dev);
   return cudaGetLastError();
 }
 

@@ -109,8 +109,20 @@ struct PauliChebArgs {
   uint32_t out_mode, acc_mode;
   double a0r, a0i, akr, aki;
 };
+// lz (a Lanczos step, qb_pauli_ground; null for qb_pauli_evolve): kChebOutSub gives hs + osub out, and with
+// partials_dev (the step's last launch) *dot_dev = Re <cur|out> over the new out, a fixed-order reduction.
+struct PauliLanczosArgs {
+  double osub;
+  double *partials_dev, *dot_dev;
+};
 cudaError_t launch_pauli_cheb(const double2 *cur, double2 *out, double2 *acc, int local_bits, const PauliChebArgs &args,
-                              int sm_count, cudaStream_t stream);
+                              int sm_count, cudaStream_t stream, const PauliLanczosArgs *lz = nullptr);
+
+// One sweep of a Lanczos step (qb_pauli_ground) over n amplitudes of three shards in one layout: w <- w - a v, then
+// *sumsq_dev = ||w||^2 (acc null; a fixed-order reduction through partials_dev) or acc <- p acc + q w (no reduction).
+// Deterministic: the new w does not depend on acc.
+cudaError_t launch_lanczos_update(double2 *w, const double2 *v, double2 *acc, uint64_t n, double a, double p, double q,
+                                  double *partials_dev, double *sumsq_dev, int sm_count, cudaStream_t stream);
 
 // The backward pass of the adjoint gradient (qb_pauli_rot_grad) over one launch of rotations: psi and lam
 // (same layout) are walked through rotations nrot-1 .. 0; for each, grad_dev[r] = Im sum_j conj(lam_j) (P_r psi)_j,

@@ -375,6 +375,37 @@ class StateVec:
                                               cf.ctypes.data_as(C.POINTER(C.c_double)), len(xs), float(t), None))
         return self
 
+    def _pauli_ground(self, terms, coefs, tol, maxiter, vector):
+        xs, zs = pauli_masks(terms, self.n)
+        cf = np.ascontiguousarray(coefs, dtype=np.float64).reshape(-1)
+        if cf.size != xs.size:
+            raise ValueError(f"{xs.size} Pauli strings but {cf.size} coefficients")
+        maxiter = int(maxiter)
+        size = min(max(1, maxiter), 65536)  # (QB_GROUND_MAX_ITER: a larger maxiter is rejected before anything is written)
+        alpha = np.zeros(size, dtype=np.float64)
+        beta = np.zeros(size, dtype=np.float64)
+        energy, resid, niter = C.c_double(), C.c_double(), C.c_int64()
+        P64, PD = C.POINTER(C.c_uint64), C.POINTER(C.c_double)
+        capi.check(self.ctx.L.qb_pauli_ground(self._h, xs.ctypes.data_as(P64), zs.ctypes.data_as(P64),
+                                              cf.ctypes.data_as(PD), len(xs), float(tol), maxiter, int(vector),
+                                              C.byref(energy), C.byref(resid), C.byref(niter), alpha.ctypes.data_as(PD),
+                                              beta.ctypes.data_as(PD)))
+        m = niter.value
+        return energy.value, resid.value, m, alpha[:m].copy(), beta[:m].copy()
+
+    def pauli_ground(self, terms, coefs, tol: float, maxiter: int = 1000):
+        """Lanczos ground-state energy of ``H = sum_t coefs[t] P_t`` on the Krylov space of ``self``
+        (qb_pauli_ground; ``self`` keeps its value).  Terms are spelled as for ``expect_pauli``; ``coefs`` are real;
+        ``tol`` bounds the Ritz residual estimate in the units of H.  Returns ``(energy, resid, niter, alpha,
+        beta)``: the lowest Ritz value, its residual estimate, the Krylov dimension m and the m coefficients of
+        the Lanczos tridiagonal (alpha_0 .. alpha_{m-1}, beta_1 .. beta_m)."""
+        return self._pauli_ground(terms, coefs, tol, maxiter, 0)
+
+    def pauli_ground_(self, terms, coefs, tol: float, maxiter: int = 1000):
+        """As ``pauli_ground``, and ``self`` becomes the normalised Ritz vector, phased so that its overlap with
+        the old value is real and positive (in place; lazy clones keep the old value)."""
+        return self._pauli_ground(terms, coefs, tol, maxiter, 1)
+
     def norm(self) -> float:  # Algebra.hs:35-36: realPart (a <.> a), the SQUARED norm
         return self.inner(self).real
 
@@ -478,3 +509,11 @@ def pauliEvolve(terms, coefs, t: float, sv: StateVec) -> StateVec:
     """``exp(-i t H) #> sv`` with ``H = sum_t coefs[t] P_t`` as a new value; ``sv`` keeps its own (a lazy clone
     evolved in place, see StateVec.pauli_evolve_)."""
     return sv.clone().pauli_evolve_(terms, coefs, t)
+
+
+def pauliGround(terms, coefs, sv: StateVec, tol: float, maxiter: int = 1000):
+    """``(energy, x)``: the Lanczos ground-state energy of ``H = sum_t coefs[t] P_t`` from ``sv`` and its Ritz vector
+    as a new value; ``sv`` keeps its own (a lazy clone turned into the vector in place, see StateVec.pauli_ground_)."""
+    x = sv.clone()
+    energy = x.pauli_ground_(terms, coefs, tol, maxiter)[0]
+    return energy, x
